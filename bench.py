@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            our CUDA path
   python bench.py --impl reference ...                     the reference's own C hetmers on host cores
+  python bench.py ... --dump-outputs DIR                   also writes the last timed step's plot to DIR/plot.npy
 
 A "step" is one full scan (pass 1 + degree exchange + pass 2 + plot reduce = T_scan of SURVEY.md
 §8d) of one synthetic FastK table.  Workload = BASELINE.json configs[1]: synthetic diploid k=31
@@ -65,7 +66,12 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=15.0, help="target CPU time of the baseline sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the plot the last timed step computed to DIR/plot.npy (our arm only)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs: only our arm returns a plot (the reference arm writes a .smu of a sample table)")
+    return args
 
 
 def workload_name(n_gpus):
@@ -250,6 +256,17 @@ def measured_traffic(kernel, nels, grid):
         return None
 
 
+def dump_outputs(dirname, plot):
+    """DIR/plot.npy: what a caller of the scan receives, the (count sum, min count) histogram of isolated pairs,
+    as float64 [1001, 501] (exact: a cell counts at most one pair per table entry, far below 2^53).  The table is
+    generated from a fixed seed, so two builds given the same arguments can be compared cell for cell."""
+    import numpy as np
+    from smudgeplot_b200 import _lib
+    os.makedirs(dirname, exist_ok=True)
+    a = plot.cpu().numpy().reshape(_lib.SMAX + 1, _lib.PLOT_W).astype(np.float64)
+    np.save(os.path.join(dirname, "plot.npy"), a)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -343,6 +360,8 @@ def run_ours(args):
         if not args.no_e2e:
             e2e = measure_e2e(args, torch, dist, dev, multi, world, rank,
                               job if multi else None, (keys, cnt) if not multi else None)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, timed_plot)
     if multi:
         t = torch.tensor([ms_total, ms_p1], dtype=torch.float64, device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -6,6 +6,8 @@ The reference ships no golden vectors for this path (SURVEY.md §4), so these fi
 tests/test_oracle.py requires oracle/hetmers_oracle.c to reproduce each .smu byte for byte, and
 the -m gpu tests require the CUDA path to do the same.  Run from the repo root, in the build
 container (needs /root/reference):   python tests/golden/make_golden.py
+Only reference_runs.json (digests of the reference's outputs on the larger seeded tables of the GPU
+tests):   python tests/golden/make_golden.py --reference-runs
 """
 import json
 import os
@@ -140,7 +142,81 @@ def main():
     meta["_conditioning"] = cond
     with open(os.path.join(HERE, "golden.json"), "w") as f:
         json.dump(meta, f, indent=1, sort_keys=True)
+    reference_runs()
+
+
+def reference_runs():
+    """reference_runs.json: what the reference binaries write for the seeded tables of the GPU tests that
+    compare with them (tests/test_gpu_parity.py MEDIUM_CASES, CONDITIONING_CASES, EXTRACT_CASES), keyed like
+    the pytest ids.  The tests regenerate the tables from their seeds (synth gives the same table on CPU and
+    GPU); the outputs, megabytes of text, are kept as entry count, line count and sha256."""
+    import tempfile
+    sys.path.insert(0, os.path.dirname(HERE))
+    import oracle_util as ou
+    import test_gpu_parity as tp
+    if not (os.path.exists(REF) and os.path.exists(REF_EXTRACT)):
+        sys.exit("oracle/_ref/ missing: run `make -C oracle` where the reference sources exist")
+    threads = min(os.cpu_count() or 4, 64)
+    key = lambda params: "-".join(str(p) for p in params)          # noqa: E731
+    runs = {"medium": {}, "conditioning": {}, "extract": {}}
+    d = tempfile.mkdtemp(prefix="reference_runs_")
+    try:
+        for c in tp.MEDIUM_CASES:
+            k, target, ploidy, het, cov, L, seed, ref_threads = c
+            G = synth.calibrate_G(k, target, ploidy, het, cov, L)
+            keys, cnt = synth.synth_table(k, G, ploidy, het, cov, L, seed)
+            table = os.path.join(d, "medium")
+            kt = synth.write_table(table, k, keys, cnt, ibyte=3, nparts=4)
+            del keys, cnt
+            r = run_ref(table, os.path.join(d, "medium"), L, ref_threads or threads)
+            assert r.returncode == 0, r.stderr
+            smu = open(os.path.join(d, "medium.smu")).read()
+            runs["medium"][key(c)] = dict(nels=kt.nels, smu_rows=len(smu.splitlines()), smu_sha256=ou.sha256_text(smu))
+            fastk.remove_ktab(table)
+            print("medium", key(c), runs["medium"][key(c)])
+        for c in tp.CONDITIONING_CASES:
+            k, G, ploidy, seed, L = c
+            ku, cn = tp.canonical_untrimmed_table(k, G, ploidy, seed)
+            ck, cc = tp._condition_numpy(ku, cn, k, L, True, True)
+            table = os.path.join(d, "cond")
+            fastk.write_ktab(table, k, ck, cc, ibyte=3, nparts=2)
+            r = run_ref(table, os.path.join(d, "cond"), L, 4)
+            assert r.returncode == 0 and "trimmed and symmetric" in r.stderr, r.stderr
+            smu = open(os.path.join(d, "cond.smu")).read()
+            runs["conditioning"][key(c)] = dict(nels=len(cc), smu_rows=len(smu.splitlines()),
+                                                smu_sha256=ou.sha256_text(smu))
+            print("conditioning", key(c), runs["conditioning"][key(c)])
+        for c in tp.EXTRACT_CASES:
+            k, G, ploidy, seed, L = c
+            keys, cnt = synth.synth_table(k, G, ploidy, 0.02, 20 * ploidy, L, seed)
+            table = os.path.join(d, "ex")
+            kt = synth.write_table(table, k, keys, cnt, ibyte=3, nparts=3)
+            r = run_ref(table, os.path.join(d, "ex"), L, threads)
+            assert r.returncode == 0, r.stderr
+            plot = np.zeros((ou.SMAX + 1, ou.PLOT_W), dtype=np.int64)
+            for ln in open(os.path.join(d, "ex.smu")).read().splitlines():
+                m, rest, n = (int(v) for v in ln.split("\t"))
+                plot[m + rest, m] = n
+            sma = os.path.join(d, "ex.sma")
+            tp.label_sma(plot, sma)                                # the .sma the test writes from its plot
+            out = os.path.join(d, "pairs", "refx")
+            shutil.rmtree(os.path.dirname(out), ignore_errors=True)
+            os.makedirs(os.path.dirname(out))
+            r = run_ref_extract(table, sma, out, L, threads)
+            assert r.returncode == 0, r.stderr
+            lists = ou.sorted_pair_files(out)
+            assert lists
+            runs["extract"][key(c)] = dict(nels=kt.nels, pairs={lab: dict(lines=len(v), sha256=ou.sha256_lines(v))
+                                                                for lab, v in lists.items()})
+            print("extract", key(c), runs["extract"][key(c)])
+    finally:
+        shutil.rmtree(d, ignore_errors=True)
+    with open(os.path.join(HERE, "reference_runs.json"), "w") as f:
+        json.dump(runs, f, indent=1, sort_keys=True)
 
 
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] == ["--reference-runs"]:
+        reference_runs()
+    else:
+        main()

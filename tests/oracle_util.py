@@ -4,6 +4,7 @@
   * brute_force() -- SURVEY.md Appendix B, an independent 15-line definition (tiny inputs only)
 """
 import ctypes as C
+import hashlib
 import os
 import subprocess
 
@@ -32,21 +33,18 @@ def oracle_lib():
     return _lib
 
 
-REF_EXTRACT = os.path.join(ROOT, "oracle", "_ref", "extract_kmer_pairs")
-
-
 def oracle_extract(table: str, ethresh: int, sma: str, out_root: str) -> int:
     """oracle restatement of extract_kmer_pairs; 0 ok / 1 cannot open / 2 needs conditioning / 3 bad .sma"""
     return oracle_lib().oracle_extract_file(table.encode(), ethresh, sma.encode(), out_root.encode())
 
 
-def have_ref_extract():
-    return os.path.exists(REF_EXTRACT) and os.access(REF_EXTRACT, os.X_OK)
+def sha256_text(text: str) -> str:
+    """digest of an output file's text (golden/reference_runs.json holds these for outputs too large to store)"""
+    return hashlib.sha256(text.encode()).hexdigest()
 
 
-def run_ref_extract(table: str, sma: str, out_root: str, ethresh: int, threads: int = 4):
-    return subprocess.run([REF_EXTRACT, f"-e{ethresh}", f"-T{threads}", f"-o{out_root}", table, sma],
-                          capture_output=True, text=True)
+def sha256_lines(lines) -> str:
+    return sha256_text("".join(ln + "\n" for ln in lines))
 
 
 def sorted_pair_files(out_root: str):

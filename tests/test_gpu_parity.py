@@ -1,8 +1,9 @@
 """GPU parity tests (run with -m gpu on the B200 box).  Everything goes through the C ABI of
 libhetmers_b200.so (in-process via ctypes, or through the drop-in `hetmers` executable) and is
 compared bit for bit with (a) the golden .smu files written by the unmodified reference binary,
-(b) the oracle on seeded tables, (c) the reference binary itself when oracle/_ref/hetmers is
-present, and (d) size-independent properties at BASELINE.json's full size."""
+(b) the oracle on seeded tables, (c) what the reference binaries wrote for larger seeded tables
+(digests in golden/reference_runs.json), and (d) size-independent properties at BASELINE.json's full size."""
+import json
 import os
 import shutil
 import subprocess
@@ -89,35 +90,56 @@ def test_extract_executable_reproduces_reference_pair_lists(name, golden_meta, t
     assert ou.sorted_pair_files(out) == _golden_pairs(name)
 
 
-@pytest.mark.parametrize("k,G,ploidy,seed,L", [(31, 400000, 3, 41, 12), (40, 150000, 2, 42, 4)])
+def reference_run(kind, *params):
+    """what the reference binaries wrote for the seeded table of one parameter set (golden/reference_runs.json,
+    recorded by golden/make_golden.py; keyed like the pytest id)"""
+    with open(os.path.join(GOLDEN, "reference_runs.json")) as f:
+        return json.load(f)[kind]["-".join(str(p) for p in params)]
+
+
+def label_sma(plot, sma):
+    """write <sma> labelling every plotted pixel by (sum + min) % 4 (three smudges, a quarter unlabelled)
+    -> (pixmap uint16[1001,501] of smudge numbers in order of first appearance, label names in that order)"""
+    s_idx, m_idx = np.nonzero(plot[:, :_lib.FMAX] > 0)
+    pix = np.zeros((_lib.SMAX + 1, _lib.PLOT_W), dtype=np.uint16)
+    labels = ["1A1B", "2A1B", "2A2B"]
+    order = []
+    with open(sma, "w") as f:
+        f.write("covB\tcovA\tfreq\tsmudge\n")
+        for s, m in zip(s_idx.tolist(), m_idx.tolist()):
+            lab = (s + m) % 4
+            if lab < 3:
+                if labels[lab] not in order:
+                    order.append(labels[lab])
+                pix[s, m] = order.index(labels[lab]) + 1
+                f.write(f"{m}\t{s - m}\t{plot[s, m]}\t{labels[lab]}\n")
+    return pix, order
+
+
+EXTRACT_CASES = [(31, 400000, 3, 41, 12), (40, 150000, 2, 42, 4)]
+
+
+@pytest.mark.parametrize("k,G,ploidy,seed,L", EXTRACT_CASES)
 def test_extract_matches_reference_binary_and_inprocess_list(k, G, ploidy, seed, L, tmp_path):
-    """bigger seeded table: our extract_kmer_pairs vs the reference's (sorted lines), and the
+    """bigger seeded table: our extract_kmer_pairs vs the reference's (sorted lines, as digests), and the
     in-process pair list (hm_scan_extract) vs the files"""
+    want = reference_run("extract", k, G, ploidy, seed, L)
     keys, cnt = synth.synth_table(k, G, ploidy, 0.02, 20 * ploidy, L, seed, device="cuda")
     name = str(tmp_path / "t")
     kt = synth.write_table(name, k, keys, cnt, ibyte=3, nparts=3)
+    assert kt.nels == want["nels"]                                    # the table the reference read
+    sma = str(tmp_path / "ann.sma")
     with hetmers.Scan(kt) as sc:
         plot, _ = sc.run()
-        s_idx, m_idx = np.nonzero(plot[:, :_lib.FMAX] > 0)
-        pix = np.zeros((_lib.SMAX + 1, _lib.PLOT_W), dtype=np.uint16)
-        labels = ["1A1B", "2A1B", "2A2B"]
-        sma = str(tmp_path / "ann.sma")
-        with open(sma, "w") as f:
-            f.write("covB\tcovA\tfreq\tsmudge\n")
-            order = []
-            for s, m in zip(s_idx.tolist(), m_idx.tolist()):
-                lab = (s + m) % 4
-                if lab < 3:
-                    if labels[lab] not in order:
-                        order.append(labels[lab])
-                    pix[s, m] = order.index(labels[lab]) + 1
-                    f.write(f"{m}\t{s - m}\t{plot[s, m]}\t{labels[lab]}\n")
+        pix, order = label_sma(plot, sma)
         rec = sc.extract(pix)
     assert len(rec) == int(plot[pix > 0].sum())                       # one record per labelled isolated pair
     out = str(tmp_path / "kp")
     hetmers.run_extract(name, sma, o=out, t=4, e=L)
     ours = ou.sorted_pair_files(out)
     assert sum(len(v) for v in ours.values()) == len(rec)
+    assert {lab: len(v) for lab, v in ours.items()} == {lab: w["lines"] for lab, w in want["pairs"].items()}
+    assert {lab: ou.sha256_lines(v) for lab, v in ours.items()} == {lab: w["sha256"] for lab, w in want["pairs"].items()}
     dna = "acgt"
     def fmt(r):
         bases = [((int(r["key_hi"]) if p < 32 else int(r["key_lo"])) >> (62 - 2 * (p & 31))) & 3 for p in range(k)]
@@ -125,13 +147,6 @@ def test_extract_matches_reference_binary_and_inprocess_list(k, G, ploidy, seed,
     mine = {}
     for r in rec[:: max(1, len(rec) // 2000)]:                        # spot-check the in-process records
         assert fmt(r) in ours[order[int(r["smudge"]) - 1]]
-    if ou.have_ref_extract():
-        rr = ou.run_ref_extract(name, sma, str(tmp_path / "ref"), L, threads=min(os.cpu_count() or 4, 64))
-        assert rr.returncode == 0, rr.stderr
-        assert ou.sorted_pair_files(str(tmp_path / "ref")) == ours
-    else:
-        assert ou.oracle_extract(name, L, sma, str(tmp_path / "ora")) == 0
-        assert ou.sorted_pair_files(str(tmp_path / "ora")) == ours
     del mine
 
 
@@ -182,16 +197,12 @@ def _condition_numpy(ku, cn, k, L, trim, symm):
     return ku, cn
 
 
-@pytest.mark.parametrize("k,G,ploidy,seed,L", [(21, 60000, 2, 31, 6), (31, 80000, 3, 32, 12), (32, 50000, 2, 33, 5),
-                                               (40, 50000, 2, 34, 6), (12, 30000, 2, 35, 12)])
-def test_gpu_conditioning_of_canonical_untrimmed_table(k, G, ploidy, seed, L, tmp_path):
-    """a FastK-style table (canonical k-mers only, every count >= 1) is trimmed and symmetrised on
-    the GPU; the .smu must equal what the REFERENCE binary writes for the table conditioned by the
-    numpy restatement, and the -v lines must be the reference's"""
+def canonical_untrimmed_table(k, G, ploidy, seed):
+    """seeded FastK-style table: canonical k-mers only, every count >= 1 -> (keys uint64, counts uint16)"""
+    import torch
     keys, cnt = synth.synth_table(k, G, ploidy, 0.02, 40, 1, seed)          # untrimmed: counts from 1
     ku = synth.keys_to_u64_numpy(keys)
     cn = cnt.numpy().astype(np.uint16)
-    import torch
     if k > 32:
         rh, rl = synth.revcomp_long(keys[:, 0].contiguous(), keys[:, 1].contiguous(), k)
         rcb = fastk.keys_u64_to_bytes(torch.stack([rh, rl], 1).numpy().view(np.uint64), k)
@@ -200,8 +211,22 @@ def test_gpu_conditioning_of_canonical_untrimmed_table(k, G, ploidy, seed, L, tm
     kb = fastk.keys_u64_to_bytes(ku, k)
     w = kb.shape[1]
     canon = kb.view(f"S{w}").reshape(-1) <= rcb.view(f"S{w}").reshape(-1)   # x <= rc(x)
+    return ku[canon], cn[canon]
+
+
+CONDITIONING_CASES = [(21, 60000, 2, 31, 6), (31, 80000, 3, 32, 12), (32, 50000, 2, 33, 5),
+                      (40, 50000, 2, 34, 6), (12, 30000, 2, 35, 12)]
+
+
+@pytest.mark.parametrize("k,G,ploidy,seed,L", CONDITIONING_CASES)
+def test_gpu_conditioning_of_canonical_untrimmed_table(k, G, ploidy, seed, L, tmp_path):
+    """a FastK-style table (canonical k-mers only, every count >= 1) is trimmed and symmetrised on
+    the GPU; the .smu must equal what the REFERENCE binary wrote for the table conditioned by the
+    numpy restatement (recorded as a digest), and the -v lines must be the reference's"""
+    want = reference_run("conditioning", k, G, ploidy, seed, L)
+    ku, cn = canonical_untrimmed_table(k, G, ploidy, seed)
     raw = str(tmp_path / "raw")
-    fastk.write_ktab(raw, k, ku[canon], cn[canon], ibyte=3, nparts=3)
+    fastk.write_ktab(raw, k, ku, cn, ibyte=3, nparts=3)
     out = str(tmp_path / "gpu")
     r = subprocess.run([_lib.BIN_PATH, "-v", f"-e{L}", "-T4", f"-o{out}", raw], input="n\n",
                        capture_output=True, text=True)
@@ -211,18 +236,11 @@ def test_gpu_conditioning_of_canonical_untrimmed_table(k, G, ploidy, seed, L, tm
                         "\n  Making trimmed table symmetric\n"
                         "\n  Starting to count covariant pairs\n"
                         "\n  Count complete, outputting table\n")
-    ck, cc = _condition_numpy(ku[canon], cn[canon], k, L, True, True)
-    cond = str(tmp_path / "cond")
-    fastk.write_ktab(cond, k, ck, cc, ibyte=3, nparts=2)
-    if ou.have_ref():
-        rr = ou.run_ref(cond, str(tmp_path / "ref"), L, threads=4, verbose=True)
-        assert rr.returncode == 0 and "trimmed and symmetric" in rr.stderr, rr.stderr
-        want = open(str(tmp_path / "ref.smu")).read()
-    else:
-        rc, trim, symm, _ = ou.oracle_file(cond, L, str(tmp_path / "ora.smu"))
-        assert (rc, trim, symm) == (0, 1, 1)
-        want = open(str(tmp_path / "ora.smu")).read()
-    assert open(out + ".smu").read() == want and len(want) > 0
+    ck, cc = _condition_numpy(ku, cn, k, L, True, True)
+    assert len(cc) == want["nels"]                                          # the table the reference read
+    got = open(out + ".smu").read()
+    assert len(got) > 0 and len(got.splitlines()) == want["smu_rows"]
+    assert ou.sha256_text(got) == want["smu_sha256"]
     # in-process route + the conditioned table itself
     with hetmers.Scan(fastk.read_ktab(raw)) as sc:
         assert sc.examine(L) == (False, False)
@@ -232,7 +250,7 @@ def test_gpu_conditioning_of_canonical_untrimmed_table(k, G, ploidy, seed, L, tm
         k2, c2, _ = sc.download(deg=False)
         plot, _ = sc.run()
     assert np.array_equal(k2, ck) and np.array_equal(c2, cc)
-    assert hetmers.smu_text(plot) == want
+    assert hetmers.smu_text(plot) == got
 
 
 def test_gpu_conditioning_trim_only_and_symm_only(golden_meta, tmp_path):
@@ -390,7 +408,7 @@ def test_long_kmer_work_split_and_filter_widths():
     assert bool((pos >= 0).all())                       # symmetric table: every reverse complement is found
 
 
-@pytest.mark.parametrize("k,target,ploidy,het,cov,L,seed,ref_threads", [
+MEDIUM_CASES = [  # ref_threads: the reference's -T when its output was recorded (0: min(cores, 64))
     (21, 1_000_000, 2, 0.01, 40, 4, 1, 1),        # BASELINE configs[0]: reference C hetmers on 1 CPU thread
     (31, 20_000_000, 2, 0.01, 40, 12, 2, 0),      # configs[1] at 1/10 of the bench size
     (31, 30_000_000, 4, 0.01, 40, 12, 3, 0),      # stand-in for configs[2] (the real S. cerevisiae table needs
@@ -398,25 +416,24 @@ def test_long_kmer_work_split_and_filter_widths():
     (31, 12_000_000, 3, 0.01, 60, 12, 4, 0),      # configs[3] parameters (triploid cov 60) at reduced size
     (31, 12_000_000, 4, 0.02, 80, 10, 5, 0),      # configs[4] parameters (tetraploid het 2% cov 80, L=10), reduced
     (40, 5_000_000, 2, 0.01, 40, 4, 6, 0),        # FastK's default k=40: two-word keys against the reference
-])
+]
+
+
+@pytest.mark.parametrize("k,target,ploidy,het,cov,L,seed,ref_threads", MEDIUM_CASES)
 def test_medium_table_matches_reference_binary(k, target, ploidy, het, cov, L, seed, ref_threads, tmp_path):
+    """our executable's .smu == the reference binary's on the same seeded table (recorded as a digest)"""
+    want = reference_run("medium", k, target, ploidy, het, cov, L, seed, ref_threads)
     G = synth.calibrate_G(k, target, ploidy, het, cov, L)
     keys, cnt = synth.synth_table(k, G, ploidy, het, cov, L, seed, device="cuda")
     name = str(tmp_path / "t")
     kt = synth.write_table(name, k, keys, cnt, ibyte=3, nparts=4)
     assert abs(kt.nels - target) < 0.25 * target          # calibrate_G is a coarse model for ploidy > 2
+    assert kt.nels == want["nels"]                         # the table the reference read
     out = str(tmp_path / "gpu")
     hetmers.run_hetmers(name, o=out, L=L, t=4)
     got = open(out + ".smu").read()
-    if ou.have_ref():
-        r = ou.run_ref(name, str(tmp_path / "ref"), L, threads=ref_threads or min(os.cpu_count() or 4, 64))
-        assert r.returncode == 0, r.stderr
-        want = open(str(tmp_path / "ref.smu")).read()
-    else:
-        rc, *_ = ou.oracle_file(name, L, str(tmp_path / "ora.smu"))
-        assert rc == 0
-        want = open(str(tmp_path / "ora.smu")).read()
-    assert got == want and len(got) > 0
+    assert len(got) > 0 and len(got.splitlines()) == want["smu_rows"]
+    assert ou.sha256_text(got) == want["smu_sha256"]
 
 
 # ------------------------------------------------------------------ (d) full-size properties --
