@@ -299,8 +299,39 @@ int  hm_scan_extract(hm_scan *s, const uint16_t *pixmap, hm_pair_rec **out, int6
 /* one call: create + run + destroy (what bench.py's e2e leg times) */
 int  hm_hetmers_host(const hm_host_table *t, const int *dev, int n_gpus,
                      int64_t *plot, hm_scan_stats *stats);
-/* copy device arrays back for tests: any pointer may be NULL */
+/* copy device arrays back for tests: any pointer may be NULL.  A sharded scan gives the
+ * concatenation of its shards and has no incidence array (deg must be NULL).                     */
 int  hm_scan_download(hm_scan *s, uint64_t *keys, uint64_t *keys_lo, uint16_t *cnt, uint8_t *deg);
+
+/* ---- sharded placement (DESIGN.md §6): tables larger than one GPU's memory -------------------
+ * Shard r of n_shards holds only the entries of its key range [cut_r, cut_r+1) on device dev[r]; the
+ * cuts sit on boundaries of the first k/2 bases, so no run of the table is split.  The same device
+ * may carry several logical shards.  Each shard loads 1/n_shards of the part files; the key ranges
+ * are established by the first hm_scan_condition (which trims / symmetrises on the way) or, for a
+ * table that needs no conditioning, by the first scan.  On a sharded scan hm_scan_examine,
+ * hm_scan_condition, hm_scan_run / hm_scan_run_path(HM_PATH_SYMM) and hm_scan_download work;
+ * hm_scan_extract, HM_PATH_DIRECT and tables that are not strand-symmetric are HM_EUNSUPPORTED.    */
+int  hm_scan_create_sharded(const hm_host_table *t, const int *dev, int n_shards, hm_scan **out);
+/* shard r: device, index of its first entry in the concatenated table, entries, and the device bytes
+ * the library keeps for it (table arrays, bucket index, plot, scan work area).  On a replica scan:
+ * device r's full replica.                                                                         */
+int  hm_scan_shard_info(const hm_scan *s, int r, int *dev, int64_t *first_index, int64_t *n,
+                        int64_t *device_bytes);
+/* Shard cuts from a sample of m records (hi / lo key words, lo NULL for k <= 32; cnt NULL = no trim):
+ * records with count < min_count are left out, add_rc adds each record's reverse complement; cut[0]
+ * = 0 and cut[r] = the first word of the (r/n_shards)-quantile rounded down to its first k/2 bases. */
+int  hm_shard_cuts(const uint64_t *hi, const uint64_t *lo, const uint16_t *cnt, int64_t m, int kmer,
+                   int min_count, int add_rc, int n_shards, uint64_t *cut);
+/* Placement of a table of nels entries (do_symm: it will be symmetrised, up to 2 x nels) on n_gpus
+ * devices with free_bytes[g] free: a full replica on every device if one fits (with the peak of
+ * conditioning it when do_symm), else one shard per device, else neither.  Pure host arithmetic from
+ * the library's own allocation sizes; need_* (optional) = the bytes per device of either choice.   */
+int  hm_device_free_bytes(int dev, int64_t *free_bytes);     /* what device `dev` has free now */
+#define HM_PLACE_NOFIT   0
+#define HM_PLACE_REPLICA 1
+#define HM_PLACE_SHARDED 2
+int  hm_plan_placement(int kmer, int64_t nels, int do_symm, int n_gpus, const int64_t *free_bytes,
+                       int64_t *need_replica, int64_t *need_shard);
 
 /* ======================= C. FastK table files (host, plain C) ============================ */
 

@@ -24,7 +24,8 @@ ABI_SYMBOLS = [
     "hm_scan_create", "hm_prewarm", "hm_set_io_threads", "hm_scan_destroy", "hm_scan_examine", "hm_scan_condition", "hm_scan_run", "hm_hetmers_host",
     "hm_scan_run_path", "hm_scan_is_symmetric", "hm_symm_plan", "hm_symm_seeds", "hm_k_symm_fingerprint", "hm_k_symm_runscan", "hm_k_symm_runs", "hm_k_symm_resolve",
     "hm_symm_status", "hm_symm_align_cut",
-    "hm_scan_download", "hm_table_open", "hm_table_close", "hm_table_view", "hm_write_smu",
+    "hm_scan_download", "hm_scan_create_sharded", "hm_scan_shard_info", "hm_shard_cuts", "hm_plan_placement", "hm_device_free_bytes",
+    "hm_table_open", "hm_table_close", "hm_table_view", "hm_write_smu",
 ]
 
 
@@ -59,6 +60,8 @@ class SymmShards(C.Structure):
 
 
 SYMM_ASYMMETRIC, SYMM_OVERFLOW = 1, 2
+PLACE_NOFIT, PLACE_REPLICA, PLACE_SHARDED = 0, 1, 2
+EUNSUPPORTED = -6
 
 
 class PairRec(C.Structure):
@@ -141,6 +144,11 @@ def lib():
     L.hm_scan_extract.argtypes = [vp, vp, C.POINTER(C.POINTER(PairRec)), C.POINTER(i64)]
     L.hm_hetmers_host.argtypes = [C.POINTER(HostTable), C.POINTER(i32), i32, vp, C.POINTER(ScanStats)]
     L.hm_scan_download.argtypes = [vp, vp, vp, vp, vp]
+    L.hm_scan_create_sharded.argtypes = [C.POINTER(HostTable), C.POINTER(i32), i32, C.POINTER(vp)]
+    L.hm_scan_shard_info.argtypes = [vp, i32, C.POINTER(i32), C.POINTER(i64), C.POINTER(i64), C.POINTER(i64)]
+    L.hm_shard_cuts.argtypes = [vp, vp, vp, i64, i32, i32, i32, i32, C.POINTER(C.c_uint64)]
+    L.hm_device_free_bytes.argtypes = [i32, C.POINTER(i64)]
+    L.hm_plan_placement.argtypes = [i32, i64, i32, i32, C.POINTER(i64), C.POINTER(i64), C.POINTER(i64)]
     L.hm_table_open.argtypes = [C.c_char_p, C.POINTER(vp)]
     L.hm_table_close.argtypes = [vp]
     L.hm_table_close.restype = None
@@ -154,3 +162,27 @@ def lib():
 def check(rc: int):
     if rc != 0:
         raise HetmersError(rc, lib().hm_last_error().decode(errors="replace"))
+
+
+def plan_placement(kmer: int, nels: int, free_bytes, do_symm: bool = False):
+    """-> (PLACE_*, bytes per device of a replica, bytes per device of a shard) for a table of nels
+    entries on len(free_bytes) devices (hm_plan_placement)"""
+    fb = (C.c_int64 * len(free_bytes))(*[int(x) for x in free_bytes])
+    rep, shd = C.c_int64(), C.c_int64()
+    r = lib().hm_plan_placement(kmer, nels, int(do_symm), len(free_bytes), fb, C.byref(rep), C.byref(shd))
+    if r < 0:
+        check(r)
+    return r, rep.value, shd.value
+
+
+def shard_cuts(hi, lo, cnt, kmer: int, n_shards: int, min_count: int = 0, add_rc: bool = False):
+    """cut keys of n_shards run-aligned key ranges from a sample of records (hm_shard_cuts): uint64[n_shards]"""
+    import numpy as np
+    hi = np.ascontiguousarray(hi, dtype=np.uint64)
+    lo = None if lo is None else np.ascontiguousarray(lo, dtype=np.uint64)
+    cnt = None if cnt is None else np.ascontiguousarray(cnt, dtype=np.uint16)
+    out = (C.c_uint64 * n_shards)()
+    check(lib().hm_shard_cuts(hi.ctypes.data, None if lo is None else lo.ctypes.data,
+                              None if cnt is None else cnt.ctypes.data, hi.size, kmer, min_count, int(add_rc),
+                              n_shards, out))
+    return np.array(out[:], dtype=np.uint64)

@@ -20,9 +20,11 @@
 #include <cub/cub.cuh>
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <string.h>
 
 #include "hetmers_b200.h"
 #include "hm_internal.h"
+#include "hm_device.cuh"
 
 __device__ __forceinline__ uint64_t rev2_64(uint64_t x)       /* reverse the 32 2-bit fields */
 { x = ((x >> 2)  & 0x3333333333333333ull) | ((x & 0x3333333333333333ull) << 2);
@@ -137,6 +139,54 @@ struct Scratch
     void free_now(void *q) { if (q != NULL) { release(q); cudaFree(q); } }
   };
 
+/* Sort (h0, l0, c0)[0,m) by key (stable: of equal keys the one nearer the front wins) and keep the
+ * first entry of every run of equal keys, back in h0 / l0 / c0; *nsel = entries kept.  l0 is NULL for
+ * k <= 32.  The second buffers come from S and are released before returning.                     */
+static int sort_unique(int kmer, uint64_t *h0, uint64_t *l0, uint16_t *c0, int64_t m, Scratch &S,
+                       int64_t *d_nsel, int64_t *nsel, void **tmp, size_t *tmp_bytes, cudaStream_t st)
+{ const int two = (l0 != NULL);
+  uint64_t *h1 = NULL, *l1 = NULL;
+  uint16_t *c1 = NULL;
+  uint8_t  *flag = NULL;
+  int       rc;
+  HM_CUDA(S.alloc(&h1,sizeof(uint64_t)*(size_t) (m+1)));
+  HM_CUDA(S.alloc(&c1,sizeof(uint16_t)*(size_t) (m+1)));
+  if (two)
+    HM_CUDA(S.alloc(&l1,sizeof(uint64_t)*(size_t) (m+1)));
+  if (!two)
+    { int bb = kmer < 32 ? 64-2*kmer : 0;
+      if ((rc = sort_pairs(h0,h1,c0,c1,m,bb,64,tmp,tmp_bytes,st)) != HM_OK) return rc;
+    }
+  else
+    { uint32_t *i0 = NULL, *i1 = NULL;
+      HM_CUDA(S.alloc(&i0,sizeof(uint32_t)*(size_t) m));
+      HM_CUDA(S.alloc(&i1,sizeof(uint32_t)*(size_t) m));
+      iota_kernel<<<GRID(m),256,0,st>>>(i0,m);
+      int bb = kmer < 64 ? 128-2*kmer : 0;
+      /* least significant word first, then a stable sort on the most significant word */
+      if ((rc = sort_pairs(l0,l1,i0,i1,m,bb,64,tmp,tmp_bytes,st)) != HM_OK) return rc;
+      gather_kernel<uint64_t><<<GRID(m),256,0,st>>>(h0,i1,m,h1);          /* hi in lo-order   */
+      if ((rc = sort_pairs(h1,l1,i1,i0,m,0,64,tmp,tmp_bytes,st)) != HM_OK) return rc;
+      /* l1 = sorted hi, i0 = final permutation */
+      gather_kernel<uint64_t><<<GRID(m),256,0,st>>>(l0,i0,m,h1);          /* h1 := lo sorted  */
+      gather_kernel<uint16_t><<<GRID(m),256,0,st>>>(c0,i0,m,c1);
+      /* arrange as (h1 = hi, l1 = lo) */
+      uint64_t *t = h1; h1 = l1; l1 = t;
+      HM_CUDA(cudaStreamSynchronize(st));
+      S.free_now(i0); S.free_now(i1);
+    }
+  /* unique (first of every run of equal keys wins) back into h0/l0/c0 */
+  HM_CUDA(S.alloc(&flag,(size_t) m));
+  first_of_run_kernel<<<GRID(m),256,0,st>>>(h1,two ? l1 : NULL,m,flag);
+  if ((rc = select_flagged(h1,flag,h0,m,d_nsel,tmp,tmp_bytes,st)) != HM_OK) return rc;
+  if (two && (rc = select_flagged(l1,flag,l0,m,d_nsel,tmp,tmp_bytes,st)) != HM_OK) return rc;
+  if ((rc = select_flagged(c1,flag,c0,m,d_nsel,tmp,tmp_bytes,st)) != HM_OK) return rc;
+  HM_CUDA(cudaMemcpyAsync(nsel,d_nsel,sizeof(int64_t),cudaMemcpyDeviceToHost,st));
+  HM_CUDA(cudaStreamSynchronize(st));
+  S.free_now(flag); S.free_now(h1); S.free_now(l1); S.free_now(c1);
+  return HM_OK;
+}
+
 /* Replace (*pk, *pl, *pc, *pn) by the conditioned table (new cudaMalloc'ed arrays with one spare
  * element).  *pl is NULL for k <= 32.  The caller's arrays are freed and replaced only when the whole
  * call has succeeded; on any failure they are untouched and every temporary is released.        */
@@ -180,52 +230,19 @@ int hm_condition_arrays(int kmer, int ethresh, int do_trim, int do_symm,
 
   if (do_symm && n > 0)
     { int64_t   m = 2*n;
-      uint64_t *h0 = NULL, *l0 = NULL, *h1 = NULL, *l1 = NULL;
-      uint16_t *c0 = NULL, *c1 = NULL;
+      uint64_t *h0 = NULL, *l0 = NULL;
+      uint16_t *c0 = NULL;
       CK(S.alloc(&h0,sizeof(uint64_t)*(size_t) (m+1)));
-      CK(S.alloc(&h1,sizeof(uint64_t)*(size_t) (m+1)));
       CK(S.alloc(&c0,sizeof(uint16_t)*(size_t) (m+1)));
-      CK(S.alloc(&c1,sizeof(uint16_t)*(size_t) (m+1)));
       if (two)
-        { CK(S.alloc(&l0,sizeof(uint64_t)*(size_t) (m+1)));
-          CK(S.alloc(&l1,sizeof(uint64_t)*(size_t) (m+1)));
-        }
+        CK(S.alloc(&l0,sizeof(uint64_t)*(size_t) (m+1)));
       append_revcomp_kernel<<<GRID(n),256,0,st>>>(ck,cl,cc,n,kmer,h0,l0,c0);
       if (own)                                       /* the trimmed intermediate is ours: drop it now */
         { CK(cudaStreamSynchronize(st));
           S.free_now(ck); S.free_now(cc); S.free_now(cl);
           ck = NULL; cc = NULL; cl = NULL; own = 0;
         }
-      if (!two)
-        { int bb = kmer < 32 ? 64-2*kmer : 0;
-          RC(sort_pairs(h0,h1,c0,c1,m,bb,64,&tmp,&tmp_bytes,st));
-        }
-      else
-        { uint32_t *i0 = NULL, *i1 = NULL;
-          CK(S.alloc(&i0,sizeof(uint32_t)*(size_t) m));
-          CK(S.alloc(&i1,sizeof(uint32_t)*(size_t) m));
-          iota_kernel<<<GRID(m),256,0,st>>>(i0,m);
-          int bb = kmer < 64 ? 128-2*kmer : 0;
-          /* least significant word first, then a stable sort on the most significant word */
-          RC(sort_pairs(l0,l1,i0,i1,m,bb,64,&tmp,&tmp_bytes,st));
-          gather_kernel<uint64_t><<<GRID(m),256,0,st>>>(h0,i1,m,h1);          /* hi in lo-order   */
-          RC(sort_pairs(h1,l1,i1,i0,m,0,64,&tmp,&tmp_bytes,st));
-          /* l1 = sorted hi, i0 = final permutation */
-          gather_kernel<uint64_t><<<GRID(m),256,0,st>>>(l0,i0,m,h1);          /* h1 := lo sorted  */
-          gather_kernel<uint16_t><<<GRID(m),256,0,st>>>(c0,i0,m,c1);
-          /* arrange as (h1 = hi, l1 = lo) */
-          uint64_t *t = h1; h1 = l1; l1 = t;
-          CK(cudaStreamSynchronize(st));
-          S.free_now(i0); S.free_now(i1);
-        }
-      /* unique (first of every run of equal keys wins) back into h0/l0/c0 */
-      CK(S.alloc(&flag,(size_t) m));
-      first_of_run_kernel<<<GRID(m),256,0,st>>>(h1,two ? l1 : NULL,m,flag);
-      RC(select_flagged(h1,flag,h0,m,d_nsel,&tmp,&tmp_bytes,st));
-      if (two) RC(select_flagged(l1,flag,l0,m,d_nsel,&tmp,&tmp_bytes,st));
-      RC(select_flagged(c1,flag,c0,m,d_nsel,&tmp,&tmp_bytes,st));
-      CK(cudaMemcpyAsync(&nsel,d_nsel,sizeof(int64_t),cudaMemcpyDeviceToHost,st));
-      CK(cudaStreamSynchronize(st));
+      RC(sort_unique(kmer,h0,l0,c0,m,S,d_nsel,&nsel,&tmp,&tmp_bytes,st));
       ck = h0; cc = c0; cl = l0; n = nsel; own = 1;
     }
 
@@ -239,5 +256,102 @@ int hm_condition_arrays(int kmer, int ethresh, int do_trim, int do_symm,
       *pk = ck; *pc = cc; *pl = cl;
     }
   *pn = n;
+  return HM_OK;
+}
+
+/* Sort + deduplicate a table held in (k, l, c)[0,*pn) (cudaMalloc'ed; l NULL for k <= 32) in place:
+ * what each shard of a sharded table does with the entries it received (originals ahead of reverse
+ * complements, so that of two equal keys the original survives, as in hm_condition_arrays).        */
+int hm_sort_unique_arrays(int kmer, uint64_t *k, uint64_t *l, uint16_t *c, int64_t *pn, cudaStream_t st)
+{ int64_t m = *pn, nsel = 0, *d_nsel = NULL;
+  void   *tmp = NULL;
+  size_t  tmp_bytes = 0;
+  if (m <= 0)
+    return HM_OK;
+  if (l != NULL && m >= 0xFFFFFFF0ll)
+    return hm_set_error(HM_EUNSUPPORTED,"a shard of %lld entries of k=%d needs 64-bit sort indices",(long long) m,kmer);
+  Scratch S;
+  HM_CUDA(S.alloc(&d_nsel,sizeof(int64_t)));
+  int rc = sort_unique(kmer,k,l,c,m,S,d_nsel,&nsel,&tmp,&tmp_bytes,st);
+  if (tmp) cudaFree(tmp);
+  if (rc == HM_OK)
+    *pn = nsel;
+  return rc;
+}
+
+/* ---- sharded placement: every entry to the shard that owns its key range ----------------------
+ * Shard r owns the keys whose first word is in [cut[r], cut[r+1]) (cut[0] = 0, ties to the higher
+ * shard, the rule owner_of() of hm_symm.cu applies); the cuts sit on boundaries of the first k/2
+ * bases, so no run of the table is split.  One thread per entry: trim by count, the entry and (when
+ * symmetrising) its reverse complement go to slot 2*owner + (0 original | 1 reverse complement).
+ * d_cursor[2*S]: count mode (okeys == NULL) adds the number of entries per slot; fill mode starts
+ * from each slot's offset in the outbox and writes the entries there (order inside a slot is free:
+ * the owner sorts).  One atomic per warp and slot.                                                */
+struct PartCuts { uint64_t c[HM_MAX_SHARDS]; };
+
+template <int KW>
+__global__ void __launch_bounds__(256)
+partition_kernel(const uint64_t *__restrict__ keys, const uint64_t *__restrict__ keys_lo,
+                 const uint16_t *__restrict__ cnt, int64_t n, int kmer, int ethresh, int do_trim, int do_symm,
+                 const PartCuts C, int S, unsigned long long *__restrict__ cursor,
+                 uint64_t *__restrict__ okeys, uint64_t *__restrict__ okeys_lo, uint16_t *__restrict__ ocnt)
+{ const unsigned FULL = 0xffffffffu;
+  const int      lane = threadIdx.x & 31;
+  const unsigned lt   = (1u << lane) - 1;
+  const int64_t  i    = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
+  uint64_t x = 0, xl = 0;
+  uint16_t c = 0;
+  bool keep = false;
+  if (i < n)
+    { x = keys[i]; c = cnt[i];
+      if (KW == 2) xl = keys_lo[i];
+      keep = !do_trim || (int) c >= ethresh;
+    }
+  for (int kind = 0; kind < 2; kind++)
+    { uint64_t y = x, yl = xl;
+      if (kind == 1)
+        revcomp_kmer<KW>(x,xl,kmer,y,yl);
+      const bool act = keep && (kind == 0 || do_symm);
+      int slot = -1;
+      if (act)
+        { int o = 0;
+#pragma unroll
+          for (int r = 1; r < HM_MAX_SHARDS; r++)            /* (a fixed trip count keeps C in the parameter bank) */
+            if (r < S)
+              o += (y >= C.c[r]);
+          slot = 2*o + kind;
+        }
+      const unsigned peers  = __match_any_sync(FULL,slot);
+      const int      leader = __ffs(peers)-1;
+      unsigned long long base = 0;
+      if (act && lane == leader)
+        base = atomicAdd(cursor+slot,(unsigned long long) __popc(peers));
+      base = __shfl_sync(FULL,base,leader);
+      if (act && okeys != NULL)
+        { const unsigned long long at = base + __popc(peers & lt);
+          okeys[at] = y; ocnt[at] = c;
+          if (KW == 2) okeys_lo[at] = yl;
+        }
+    }
+}
+
+int hm_k_partition(const uint64_t *keys, const uint64_t *keys_lo, const uint16_t *cnt, int64_t n, int kmer,
+                   int ethresh, int do_trim, int do_symm, const uint64_t *cut, int n_shards,
+                   unsigned long long *d_cursor, uint64_t *okeys, uint64_t *okeys_lo, uint16_t *ocnt,
+                   cudaStream_t st)
+{ if (n_shards < 1 || n_shards > HM_MAX_SHARDS || kmer < 1 || kmer > HM_MAX_KMER || (kmer > 32) != (keys_lo != NULL))
+    return hm_set_error(HM_EINVAL,"partition: bad arguments");
+  if (n <= 0)
+    return HM_OK;
+  PartCuts C;
+  memset(&C,0,sizeof(C));
+  for (int r = 0; r < n_shards; r++) C.c[r] = cut[r];
+  if (kmer <= 32)
+    partition_kernel<1><<<GRID(n),256,0,st>>>(keys,NULL,cnt,n,kmer,ethresh,do_trim,do_symm,C,n_shards,d_cursor,okeys,NULL,ocnt);
+  else
+    partition_kernel<2><<<GRID(n),256,0,st>>>(keys,keys_lo,cnt,n,kmer,ethresh,do_trim,do_symm,C,n_shards,d_cursor,okeys,okeys_lo,ocnt);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess)
+    return hm_cuda_fail(e,"partition_kernel");
   return HM_OK;
 }

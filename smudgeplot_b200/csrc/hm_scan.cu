@@ -6,8 +6,10 @@
  *   hm_scan_examine  trimmed? / symmetric? decisions of examine_table (PloidyPlot.c:1167-1230)
  *   hm_scan_run      pass 1 -> (degree exchange when >1 GPU) -> pass 2 -> plot D2H  ("T_scan")
  *
- * Every device holds a full replica of the table (180 GB HBM3e holds 16e9 k=31 entries); work is
- * sharded by contiguous index range [lo_g, hi_g).  With one GPU there is no exchange at all.
+ * Every device holds a full replica of the table whenever one fits; work is sharded by contiguous
+ * index range [lo_g, hi_g).  With one GPU there is no exchange at all.  A table too large for one
+ * device is placed SHARDED instead (hm_scan_create_sharded, DESIGN.md §6): device g keeps only the
+ * entries [lo_g, hi_g) of its run-aligned key range, at local index 0.
  * With several GPUs in this single process the loader gathers the shards over NVLink peer
  * copies and foreign degree bytes are reached through the owner's array (remote atomics / loads
  * fused into the two kernels; summed by a peer-memory kernel of hm_peer.cu if there are no
@@ -64,6 +66,9 @@ struct hm_scan
     int      have_symm;                   /* symmetric-scan work areas allocated, cuts aligned              */
     int      last_path;                   /* HM_PATH_DIRECT / HM_PATH_SYMM of the last run                  */
     int      invalid;                     /* a failed conditioning left the replicas inconsistent            */
+    int      sharded;                     /* d[r] holds only entries [d[r].lo, d[r].hi), at local index 0   */
+    int      aligned;                     /* sharded: shard r owns the keys in [cut[r], cut[r+1]) (run-aligned) */
+    uint64_t cut[HM_MAX_GPUS];
     hm_symm_shards ssh[HM_MAX_GPUS];
     uint64_t seed[2];
   };
@@ -285,7 +290,7 @@ static int is_pageable(const void *p)
  * staging buffers and unpacks them on st (copy of chunk c+1 overlaps the unpack of chunk c);
  * pageable sources additionally go through two pinned host buffers filled by host threads.      */
 static int load_range(hm_scan *s, DevTable *D, const hm_host_table *t, const int64_t *d_index,
-                      int64_t first, int64_t count)
+                      int64_t first, int64_t count, int64_t base)
 { int      kbyte = (t->kmer+3)>>2;
   int      pbyte = kbyte - t->ibyte + 2;
   uint8_t *stage[2] = { NULL, NULL };
@@ -318,7 +323,7 @@ static int load_range(hm_scan *s, DevTable *D, const hm_host_table *t, const int
     }
   /* one GPU: the whole table arrives here in order, so the bucket index is built chunk by chunk
    * right behind the unpack (hidden behind the next chunk's H2D); so is the symmetry fingerprint   */
-  const int inc = (s->ngpu == 1 && first == 0 && count == s->n);
+  const int inc = (!s->sharded && s->ngpu == 1 && first == 0 && count == s->n);
   HM_CUDA(cudaStreamSynchronize(D->st));         /* (pool) allocations are used on both streams */
   int64_t pstart = 0;                               /* ordinal of the part's first record */
   for (int p = 0; p < t->nparts && rc == HM_OK; p++)
@@ -349,8 +354,8 @@ static int load_range(hm_scan *s, DevTable *D, const hm_host_table *t, const int
           if (e != cudaSuccess) { rc = hm_cuda_fail(e,"cudaMemcpyAsync(H2D records)"); break; }
           cudaEventRecord(copied[b],D->st_copy);
           cudaStreamWaitEvent(D->st,copied[b],0);
-          rc = hm_k_unpack_records(stage[b],m,o,d_index,t->ibyte,t->kmer,D->keys+o,
-                                   D->keys_lo ? D->keys_lo+o : NULL,D->cnt+o,D->st);
+          rc = hm_k_unpack_records(stage[b],m,o,d_index,t->ibyte,t->kmer,D->keys+(o-base),
+                                   D->keys_lo ? D->keys_lo+(o-base) : NULL,D->cnt+(o-base),D->st);
           __sync_fetch_and_add(&s->launches,1);
           cudaEventRecord(unpacked[b],D->st);
           if (inc && rc == HM_OK)
@@ -358,7 +363,7 @@ static int load_range(hm_scan *s, DevTable *D, const hm_host_table *t, const int
               __sync_fetch_and_add(&s->launches,1);
             }
           if (rc == HM_OK && s->kmer >= HM_SYMM_MIN_KMER)       /* symmetry fingerprint of what this device loads */
-            { rc = hm_k_symm_fingerprint(D->keys,D->keys_lo,D->cnt,o,o+m,s->kmer,s->seed,D->fp_acc,D->st);
+            { rc = hm_k_symm_fingerprint(D->keys,D->keys_lo,D->cnt,o-base,o-base+m,s->kmer,s->seed,D->fp_acc,D->st);
               __sync_fetch_and_add(&s->launches,1);
             }
           used[b] = 1;
@@ -398,7 +403,7 @@ static void *load_worker(void *arg)
   if (e != cudaSuccess)
     J->rc = hm_cuda_fail(e,"stub index upload");
   else
-    J->rc = load_range(s,D,J->t,d_index,D->lo,D->hi-D->lo);
+    J->rc = load_range(s,D,J->t,d_index,D->lo,D->hi-D->lo,s->sharded ? D->lo : 0);
   if (d_index != NULL) dfree(D->dev,D->st,d_index);
   if (J->rc != HM_OK)
     { strncpy(J->msg,hm_last_error(),sizeof(J->msg)-1); J->msg[sizeof(J->msg)-1] = 0; }
@@ -421,7 +426,7 @@ static int fingerprint_verdict(hm_scan *s)
   return HM_OK;
 }
 
-extern "C" int hm_scan_create(const hm_host_table *t, const int *dev, int n_gpus, hm_scan **out)
+static int create_scan(const hm_host_table *t, const int *dev, int n_gpus, int sharded, hm_scan **out)
 { double t0 = now_ms();
   if (t == NULL || out == NULL || n_gpus < 1 || n_gpus > HM_MAX_GPUS)
     return hm_set_error(HM_EINVAL,"hm_scan_create: bad arguments");
@@ -439,9 +444,12 @@ extern "C" int hm_scan_create(const hm_host_table *t, const int *dev, int n_gpus
   if (s == NULL)
     return hm_set_error(HM_ENOMEM,"out of host memory");
   s->kmer = t->kmer; s->ibyte = t->ibyte; s->n = t->nels; s->ngpu = n_gpus;
+  s->sharded = sharded;
   s->bits  = hm_pick_bucket_bits(s->n);
   s->fpos  = hm_pick_filter_bits(s->n);
   s->idx64 = (s->n >= 0xFFFFFFF0ll);
+  if (sharded)                                     /* bucket offsets are local to a shard */
+    s->idx64 = ((s->n+n_gpus-1)/n_gpus >= 0xFFFFFFF0ll);
   hm_symm_seeds(s->seed);
   int64_t n  = s->n;
   size_t  ib = s->idx64 ? 8 : 4;
@@ -457,16 +465,17 @@ extern "C" int hm_scan_create(const hm_host_table *t, const int *dev, int n_gpus
       D->dev = dev ? dev[g] : g;
       D->lo  = n*g/n_gpus;
       D->hi  = n*(g+1)/n_gpus;
+      int64_t na = sharded ? D->hi-D->lo : n;            /* entries held on this device */
       cudaError_t e;
 #define TRY(call) if (rc == HM_OK && (e = (call)) != cudaSuccess) rc = hm_cuda_fail(e,#call)
       TRY(cudaSetDevice(D->dev));
-      pool_setup(D->dev,n_gpus == 1);
+      pool_setup(D->dev,n_gpus == 1 && !sharded);
       TRY(cudaStreamCreateWithFlags(&D->st,cudaStreamNonBlocking));
       TRY(cudaStreamCreateWithFlags(&D->st_copy,cudaStreamNonBlocking));
-      TRY(dalloc(D->dev,D->st,(void **) &D->keys,sizeof(uint64_t)*(size_t) (n+1)));
+      TRY(dalloc(D->dev,D->st,(void **) &D->keys,sizeof(uint64_t)*(size_t) (na+1)));
       if (t->kmer > 32)
-        TRY(dalloc(D->dev,D->st,(void **) &D->keys_lo,sizeof(uint64_t)*(size_t) (n+1)));
-      TRY(dalloc(D->dev,D->st,(void **) &D->cnt,sizeof(uint16_t)*(size_t) (n+8)));
+        TRY(dalloc(D->dev,D->st,(void **) &D->keys_lo,sizeof(uint64_t)*(size_t) (na+1)));
+      TRY(dalloc(D->dev,D->st,(void **) &D->cnt,sizeof(uint16_t)*(size_t) (na+8)));
       TRY(dalloc(D->dev,D->st,(void **) &D->bucket,ib*(((size_t) 1<<s->bits)+1)));
       TRY(dalloc(D->dev,D->st,(void **) &D->plot,sizeof(unsigned long long)*HM_PLOT_CELLS));
       TRY(dalloc(D->dev,D->st,(void **) &D->fp_acc,4*sizeof(uint64_t)));
@@ -495,7 +504,7 @@ extern "C" int hm_scan_create(const hm_host_table *t, const int *dev, int n_gpus
         }
     }
   double t_rec = now_ms();
-  if (n_gpus > 1 && rc == HM_OK)
+  if (n_gpus > 1 && rc == HM_OK && !sharded)
     { for (int g = 0; g < n_gpus && rc == HM_OK; g++)        /* all-gather by peer copies */
         for (int h = 0; h < n_gpus && rc == HM_OK; h++)
           if (h != g)
@@ -516,10 +525,10 @@ extern "C" int hm_scan_create(const hm_host_table *t, const int *dev, int n_gpus
       for (int g = 0; g < n_gpus; g++)
         { cudaSetDevice(s->d[g].dev); cudaStreamSynchronize(s->d[g].st); }
     }
-  for (int g = 0; g < n_gpus && rc == HM_OK && n_gpus > 1; g++)     /* (one GPU: done chunk-wise) */
+  for (int g = 0; g < n_gpus && rc == HM_OK && (n_gpus > 1 || sharded); g++)     /* (one GPU: done chunk-wise) */
     { DevTable *D = s->d+g;
       cudaSetDevice(D->dev);
-      rc = hm_k_build_bucket_index(D->keys,n,s->bits,D->bucket,s->idx64,D->st);
+      rc = hm_k_build_bucket_index(D->keys,sharded ? D->hi-D->lo : n,s->bits,D->bucket,s->idx64,D->st);
       s->launches += 1;
     }
   for (int g = 0; g < n_gpus; g++)
@@ -534,6 +543,388 @@ extern "C" int hm_scan_create(const hm_host_table *t, const int *dev, int n_gpus
   s->ms_load = now_ms()-t0;
   s->ms_alloc = t_alloc-t0; s->ms_records = t_rec-t_alloc; s->ms_index = now_ms()-t_rec;
   *out = s;
+  return HM_OK;
+}
+
+extern "C" int hm_scan_create(const hm_host_table *t, const int *dev, int n_gpus, hm_scan **out)
+{ return create_scan(t,dev,n_gpus,0,out); }
+
+extern "C" int hm_scan_create_sharded(const hm_host_table *t, const int *dev, int n_shards, hm_scan **out)
+{ if (t != NULL && t->kmer < HM_SYMM_MIN_KMER)
+    return hm_set_error(HM_EUNSUPPORTED,"a sharded table needs k >= %d (k=%d)",HM_SYMM_MIN_KMER,t->kmer);
+  if (n_shards > HM_MAX_SHARDS)
+    return hm_set_error(HM_EINVAL,"hm_scan_create_sharded: at most %d shards",HM_MAX_SHARDS);
+  return create_scan(t,dev,n_shards,1,out);
+}
+
+/* reverse complement of a left-aligned packed k-mer (k <= 32) */
+static uint64_t revcomp64(uint64_t x, int k)
+{ x = ~x;
+  x = ((x >> 2)  & 0x3333333333333333ull) | ((x & 0x3333333333333333ull) << 2);
+  x = ((x >> 4)  & 0x0F0F0F0F0F0F0F0Full) | ((x & 0x0F0F0F0F0F0F0F0Full) << 4);
+  x = ((x >> 8)  & 0x00FF00FF00FF00FFull) | ((x & 0x00FF00FF00FF00FFull) << 8);
+  x = ((x >> 16) & 0x0000FFFF0000FFFFull) | ((x & 0x0000FFFF0000FFFFull) << 16);
+  x = (x >> 32) | (x << 32);
+  if (k < 32)
+    x = (x & (((uint64_t) 1 << (2*k))-1)) << (64-2*k);
+  return x;
+}
+
+/* reverse complement of a left-aligned packed k-mer of 33..64 bases held in two words */
+static void revcomp128(uint64_t hi, uint64_t lo, int k, uint64_t *rhi, uint64_t *rlo)
+{ /* reversing all 64 slots swaps the words; the k real bases end up right-aligned over 128 bits */
+  uint64_t a = revcomp64(lo,32), b = revcomp64(hi,32);      /* full-word reverse complements */
+  int      sh = 2*(64-k);                                    /* pad slots now sit on top: shift them out */
+  if (sh == 0) { *rhi = a; *rlo = b; }
+  else         { *rhi = (a << sh) | (b >> (64-sh)); *rlo = b << sh; }
+}
+
+/* ---- sharded placement (DESIGN.md §6) --------------------------------------------------------- */
+
+static int cmp_u64(const void *a, const void *b)
+{ uint64_t x = *(const uint64_t *) a, y = *(const uint64_t *) b;
+  return x < y ? -1 : (x > y);
+}
+
+extern "C" int hm_shard_cuts(const uint64_t *hi, const uint64_t *lo, const uint16_t *cnt, int64_t m, int kmer,
+                             int min_count, int add_rc, int n_shards, uint64_t *cut)
+{ if (hi == NULL || cut == NULL || m < 0 || n_shards < 1 || n_shards > HM_MAX_SHARDS ||
+      kmer < HM_SYMM_MIN_KMER || kmer > HM_MAX_KMER || (kmer > 32 && add_rc && lo == NULL))
+    return hm_set_error(HM_EINVAL,"hm_shard_cuts: bad arguments");
+  const uint64_t pmask = ~(uint64_t) 0 << (64-2*(kmer>>1));      /* the first k/2 bases: one run */
+  uint64_t *v = (uint64_t *) malloc(sizeof(uint64_t)*(size_t) (2*m+1));
+  if (v == NULL)
+    return hm_set_error(HM_ENOMEM,"out of host memory");
+  int64_t nv = 0;
+  for (int64_t i = 0; i < m; i++)
+    { if (cnt != NULL && (int) cnt[i] < min_count)
+        continue;
+      v[nv++] = hi[i] & pmask;
+      if (add_rc)
+        { uint64_t r, rl;
+          if (kmer > 32) revcomp128(hi[i],lo[i],kmer,&r,&rl);
+          else           r = revcomp64(hi[i],kmer);
+          v[nv++] = r & pmask;
+        }
+    }
+  qsort(v,(size_t) nv,sizeof(uint64_t),cmp_u64);
+  cut[0] = 0;
+  for (int r = 1; r < n_shards; r++)
+    cut[r] = nv > 0 ? v[nv*r/n_shards] : 0;
+  free(v);
+  return HM_OK;
+}
+
+/* Device bytes one device keeps for the symmetric scan of a table of which it holds `n` entries and
+ * scans `range` of them: table arrays, bucket index, plot, fingerprint sums and the scan's work area
+ * (candidate records and run heads for `range` entries, Bloom segments sized for n_seg x seg_n).  A
+ * replica holds all n entries and scans its run-aligned 1/G of them (ensure_symm); a shard holds
+ * and scans its own entries.                                                                      */
+static int64_t resident_bytes(int kmer, int64_t n, int64_t range, int bits, int idx64, int n_seg, int64_t seg_n)
+{ hm_symm_layout L;
+  int64_t b = (int64_t) sizeof(uint64_t)*(n+1)*(kmer > 32 ? 2 : 1) + (int64_t) sizeof(uint16_t)*(n+8)
+            + (idx64 ? 8 : 4)*(((int64_t) 1 << bits)+1) + (int64_t) sizeof(unsigned long long)*HM_PLOT_CELLS + 32;
+  if (range > seg_n*n_seg) range = seg_n*n_seg;
+  if (kmer >= HM_SYMM_MIN_KMER && hm_symm_plan(seg_n*n_seg,range,kmer,n_seg,&L) == HM_OK)
+    b += L.bytes;
+  return b;
+}
+
+/* peak of conditioning m entries into m2 on one device (replica: hm_condition_arrays; shard: raw +
+ * outbox, then inbox + its sort buffers + flags + CUB temporary storage, about one more copy)     */
+static int64_t condition_peak(int kmer, int64_t m, int64_t m2)
+{ int64_t tb = 8*(kmer > 32 ? 2 : 1) + 2;
+  int64_t a = tb*(m+m2);
+  int64_t b = 3*tb*m2 + (kmer > 32 ? 8*m2 : 0) + m2;
+  return a > b ? a : b;
+}
+
+/* entries a shard may receive: for k > 32 its sort carries a 32-bit permutation (hm_sort_unique_arrays) */
+#define SHARD_SORT_MAX 0xFFFFFFF0ll
+
+extern "C" int hm_plan_placement(int kmer, int64_t nels, int do_symm, int n_gpus, const int64_t *free_bytes,
+                                 int64_t *need_replica, int64_t *need_shard)
+{ if (kmer < 1 || kmer > HM_MAX_KMER || nels < 0 || n_gpus < 1 || n_gpus > HM_MAX_SHARDS || free_bytes == NULL)
+    return hm_set_error(HM_EINVAL,"hm_plan_placement: bad arguments");
+  const int     G = n_gpus;
+  const int64_t n2 = do_symm ? 2*nels : nels;          /* entries after conditioning (at most) */
+  int64_t fmin = free_bytes[0];
+  for (int g = 1; g < G; g++)
+    if (free_bytes[g] < fmin) fmin = free_bytes[g];
+  /* a replica: the whole table on every device, each scanning its run-aligned 1/G (+ slack for the
+   * alignment); symmetrising it in place first (hm_condition_arrays) peaks above that               */
+  int64_t rng = (n2+G-1)/G;
+  rng += rng/20 + 1024;
+  int64_t rep = resident_bytes(kmer,n2,rng,hm_pick_bucket_bits(n2),n2 >= 0xFFFFFFF0ll,G,(n2+G-1)/G);
+  if (do_symm)
+    { int64_t pk = resident_bytes(kmer,nels,0,hm_pick_bucket_bits(nels),nels >= 0xFFFFFFF0ll,1,nels) + condition_peak(kmer,nels,n2);
+      if (pk > rep) rep = pk;
+      if (kmer > 32 && n2 >= 0xFFFFFFF0ll)             /* beyond hm_condition_arrays' 32-bit sort indices */
+        rep = INT64_MAX;
+    }
+  /* a shard: its 1/S share with 5 % slack for the sampled cuts, the bucket index of the whole table's width */
+  int64_t per = (nels+G-1)/G, per2 = (n2+G-1)/G;
+  per2 += per2/20 + 1024;
+  int     bits = hm_pick_bucket_bits(n2);
+  int64_t fix = (per2 >= 0xFFFFFFF0ll ? 8 : 4)*(((int64_t) 1 << bits)+1) + (int64_t) sizeof(unsigned long long)*HM_PLOT_CELLS;
+  int64_t shd = resident_bytes(kmer,per2,per2,bits,per2 >= 0xFFFFFFF0ll,G,per2);
+  if (fix + condition_peak(kmer,per,per2) > shd)          /* the redistribution, before the scan's work area exists */
+    shd = fix + condition_peak(kmer,per,per2);
+  if (kmer > 32 && per2 >= SHARD_SORT_MAX)
+    shd = INT64_MAX;
+  if (need_replica) *need_replica = rep;
+  if (need_shard)   *need_shard = shd;
+  if (rep <= fmin)  return HM_PLACE_REPLICA;
+  if (G > 1 && shd <= fmin) return HM_PLACE_SHARDED;
+  return HM_PLACE_NOFIT;
+}
+
+extern "C" int hm_device_free_bytes(int dev, int64_t *free_bytes)
+{ size_t fr = 0, tot = 0;
+  if (free_bytes == NULL)
+    return hm_set_error(HM_EINVAL,"hm_device_free_bytes: no output");
+  int cur = 0;
+  cudaGetDevice(&cur);
+  HM_CUDA(cudaSetDevice(dev));
+  cudaError_t e = cudaMemGetInfo(&fr,&tot);
+  cudaSetDevice(cur);
+  if (e != cudaSuccess)
+    return hm_cuda_fail(e,"cudaMemGetInfo");
+  *free_bytes = (int64_t) fr;
+  return HM_OK;
+}
+
+/* Give every shard the run-aligned key range [cut[r], cut[r+1]) -- trimming (count >= ethresh) and
+ * adding reverse complements on the way when asked: sample -> cuts (host) -> partition_kernel
+ * counts, then fills per-owner outboxes -> peer copies into each owner's inbox (originals first) ->
+ * sort + first-of-run per owner -> bucket index + fingerprint per shard.                         */
+typedef struct { int dev, kmer, rc; cudaStream_t st; uint64_t *k, *l; uint16_t *c; int64_t *n; char msg[512]; } SortJob;
+
+static void *sort_worker(void *arg)
+{ SortJob *J = (SortJob *) arg;
+  cudaError_t e = cudaSetDevice(J->dev);
+  J->rc = (e != cudaSuccess) ? hm_cuda_fail(e,"cudaSetDevice") : hm_sort_unique_arrays(J->kmer,J->k,J->l,J->c,J->n,J->st);
+  if (J->rc != HM_OK)
+    { strncpy(J->msg,hm_last_error(),sizeof(J->msg)-1); J->msg[sizeof(J->msg)-1] = 0; }
+  return NULL;
+}
+
+static int shard_partition(hm_scan *s, int ethresh, int do_trim, int do_symm)
+{ const int S = s->ngpu, kmer = s->kmer, two = (kmer > 32);
+  int       rc = HM_OK;
+  /* 1. cuts from an equal-stride sample of all shards */
+  const int64_t want = 1 << 15;
+  int64_t step = s->n / ((int64_t) S*want);
+  if (step < 1) step = 1;
+  int64_t ns = 0;
+  for (int r = 0; r < S; r++) ns += (s->d[r].hi-s->d[r].lo+step-1)/step;
+  uint64_t *sh = (uint64_t *) malloc(sizeof(uint64_t)*(size_t) (ns+1));
+  uint64_t *sl = (uint64_t *) malloc(sizeof(uint64_t)*(size_t) (ns+1));
+  uint16_t *sc = (uint16_t *) malloc(sizeof(uint16_t)*(size_t) (ns+1));
+  if (sh == NULL || sl == NULL || sc == NULL)
+    { free(sh); free(sl); free(sc); return hm_set_error(HM_ENOMEM,"out of host memory"); }
+  int64_t at = 0;
+  for (int r = 0; r < S && rc == HM_OK; r++)
+    { DevTable *D = s->d+r;
+      int64_t   m = (D->hi-D->lo+step-1)/step;
+      if (m <= 0) continue;
+      cudaError_t e = cudaSetDevice(D->dev);
+      if (e == cudaSuccess) e = cudaMemcpy2D(sh+at,8,D->keys,8*step,8,m,cudaMemcpyDeviceToHost);
+      if (e == cudaSuccess && two) e = cudaMemcpy2D(sl+at,8,D->keys_lo,8*step,8,m,cudaMemcpyDeviceToHost);
+      if (e == cudaSuccess) e = cudaMemcpy2D(sc+at,2,D->cnt,2*step,2,m,cudaMemcpyDeviceToHost);
+      if (e != cudaSuccess) rc = hm_cuda_fail(e,"shard sample");
+      at += m;
+    }
+  uint64_t cut[HM_MAX_SHARDS];
+  if (rc == HM_OK)
+    rc = hm_shard_cuts(sh,two ? sl : NULL,do_trim ? sc : NULL,at,kmer,ethresh,do_symm,S,cut);
+  free(sh); free(sl); free(sc);
+  if (rc != HM_OK)
+    return rc;
+
+  /* 2. count per (source, owner, kind), then fill each source's outbox */
+  typedef unsigned long long ull;
+  ull      cnts[HM_MAX_SHARDS][2*HM_MAX_SHARDS];
+  int64_t  ooff[HM_MAX_SHARDS][2*HM_MAX_SHARDS+1];        /* slot offsets inside source r's outbox */
+  ull     *d_cur[HM_MAX_SHARDS];
+  uint64_t *ok[HM_MAX_SHARDS], *ol[HM_MAX_SHARDS];
+  uint16_t *oc[HM_MAX_SHARDS];
+  memset(d_cur,0,sizeof(d_cur)); memset(ok,0,sizeof(ok)); memset(ol,0,sizeof(ol)); memset(oc,0,sizeof(oc));
+  uint64_t *ik[HM_MAX_SHARDS], *il[HM_MAX_SHARDS];
+  uint16_t *ic[HM_MAX_SHARDS];
+  memset(ik,0,sizeof(ik)); memset(il,0,sizeof(il)); memset(ic,0,sizeof(ic));
+  int64_t  inn[HM_MAX_SHARDS];
+  ull      fill_end[HM_MAX_SHARDS][2*HM_MAX_SHARDS];
+#define TRY(call) do { cudaError_t _e = (call); if (_e != cudaSuccess && rc == HM_OK) rc = hm_cuda_fail(_e,#call); } while (0)
+  /* every device works at once: each loop only enqueues, the synchronisation follows in a loop of its own */
+  for (int r = 0; r < S && rc == HM_OK; r++)
+    { DevTable *D = s->d+r;
+      TRY(cudaSetDevice(D->dev));
+      TRY(cudaMalloc(&d_cur[r],sizeof(ull)*2*S));
+      TRY(cudaMemsetAsync(d_cur[r],0,sizeof(ull)*2*S,D->st));
+      if (rc == HM_OK)
+        rc = hm_k_partition(D->keys,D->keys_lo,D->cnt,D->hi-D->lo,kmer,ethresh,do_trim,do_symm,cut,S,
+                            d_cur[r],NULL,NULL,NULL,D->st);
+      TRY(cudaMemcpyAsync(cnts[r],d_cur[r],sizeof(ull)*2*S,cudaMemcpyDeviceToHost,D->st));
+      s->launches += 1;
+    }
+  for (int r = 0; r < S; r++)
+    { cudaSetDevice(s->d[r].dev);
+      TRY(cudaStreamSynchronize(s->d[r].st));
+    }
+  for (int o = 0; o < S && rc == HM_OK; o++)               /* what every owner will receive */
+    { inn[o] = 0;
+      for (int r = 0; r < S; r++) inn[o] += (int64_t) (cnts[r][2*o] + cnts[r][2*o+1]);
+      if (two && inn[o] >= SHARD_SORT_MAX)
+        rc = hm_set_error(HM_EUNSUPPORTED,"shard %d would receive %lld entries of k=%d, more than its sort handles "
+                          "(%lld): use more shards",o,(long long) inn[o],kmer,(long long) SHARD_SORT_MAX);
+    }
+  if (rc != HM_OK)                                          /* nothing has been touched yet */
+    { for (int r = 0; r < S; r++)
+        { cudaSetDevice(s->d[r].dev); cudaFree(d_cur[r]); }
+      return rc;
+    }
+  for (int r = 0; r < S && rc == HM_OK; r++)
+    { DevTable *D = s->d+r;
+      ooff[r][0] = 0;
+      for (int j = 0; j < 2*S; j++) ooff[r][j+1] = ooff[r][j] + (int64_t) cnts[r][j];
+      int64_t tot = ooff[r][2*S];
+      TRY(cudaSetDevice(D->dev));
+      TRY(cudaMalloc(&ok[r],sizeof(uint64_t)*(size_t) (tot+1)));
+      if (two) TRY(cudaMalloc(&ol[r],sizeof(uint64_t)*(size_t) (tot+1)));
+      TRY(cudaMalloc(&oc[r],sizeof(uint16_t)*(size_t) (tot+1)));
+      TRY(cudaMemcpyAsync(d_cur[r],ooff[r],sizeof(ull)*2*S,cudaMemcpyHostToDevice,D->st));
+      if (rc == HM_OK)
+        rc = hm_k_partition(D->keys,D->keys_lo,D->cnt,D->hi-D->lo,kmer,ethresh,do_trim,do_symm,cut,S,
+                            d_cur[r],ok[r],ol[r],oc[r],D->st);
+      TRY(cudaMemcpyAsync(fill_end[r],d_cur[r],sizeof(ull)*2*S,cudaMemcpyDeviceToHost,D->st));
+      s->launches += 1;
+    }
+  for (int r = 0; r < S; r++)
+    { DevTable *D = s->d+r;
+      cudaSetDevice(D->dev);
+      TRY(cudaStreamSynchronize(D->st));
+      for (int j = 0; j < 2*S && rc == HM_OK; j++)           /* a fill that disagrees with its count */
+        if ((int64_t) fill_end[r][j] != ooff[r][j+1])
+          rc = hm_set_error(HM_ECUDA,"partition of shard %d: slot %d filled to %llu, counted %lld",r,j,
+                            fill_end[r][j],(long long) ooff[r][j+1]);
+    }
+  int raw_gone = (rc == HM_OK);
+  for (int r = 0; r < S && rc == HM_OK; r++)                /* the raw shards now live in the outboxes */
+    { DevTable *D = s->d+r;
+      cudaSetDevice(D->dev);
+      cudaFree(D->keys); cudaFree(D->keys_lo); cudaFree(D->cnt);
+      D->keys = NULL; D->keys_lo = NULL; D->cnt = NULL;
+    }
+  /* 3. every owner pulls its slots: originals of all sources first, then their reverse complements */
+  for (int o = 0; o < S && rc == HM_OK; o++)
+    { DevTable *O = s->d+o;
+      int64_t   tot = inn[o];
+      TRY(cudaSetDevice(O->dev));
+      TRY(cudaMalloc(&ik[o],sizeof(uint64_t)*(size_t) (tot+1)));
+      if (two) TRY(cudaMalloc(&il[o],sizeof(uint64_t)*(size_t) (tot+1)));
+      TRY(cudaMalloc(&ic[o],sizeof(uint16_t)*(size_t) (tot+8)));
+      int64_t dst = 0;
+      for (int kind = 0; kind < 2; kind++)
+        for (int r = 0; r < S && rc == HM_OK; r++)
+          { int64_t c = (int64_t) cnts[r][2*o+kind], src = ooff[r][2*o+kind];
+            if (c == 0) continue;
+            int sd = s->d[r].dev;
+            TRY(cudaMemcpyPeerAsync(ik[o]+dst,O->dev,ok[r]+src,sd,sizeof(uint64_t)*(size_t) c,O->st));
+            if (two) TRY(cudaMemcpyPeerAsync(il[o]+dst,O->dev,ol[r]+src,sd,sizeof(uint64_t)*(size_t) c,O->st));
+            TRY(cudaMemcpyPeerAsync(ic[o]+dst,O->dev,oc[r]+src,sd,sizeof(uint16_t)*(size_t) c,O->st));
+            dst += c;
+          }
+    }
+  for (int o = 0; o < S; o++)
+    { cudaSetDevice(s->d[o].dev);
+      TRY(cudaStreamSynchronize(s->d[o].st));
+    }
+  for (int r = 0; r < S; r++)
+    { cudaSetDevice(s->d[r].dev);
+      cudaFree(ok[r]); cudaFree(ol[r]); cudaFree(oc[r]); cudaFree(d_cur[r]);
+    }
+  /* 4. sort + first of every run, per owner: one host thread each (the sort synchronises its stream) */
+  if (rc == HM_OK)
+    { SortJob   job[HM_MAX_SHARDS];
+      pthread_t th[HM_MAX_SHARDS];
+      int       made[HM_MAX_SHARDS];
+      for (int o = 0; o < S; o++)
+        { job[o].dev = s->d[o].dev; job[o].st = s->d[o].st; job[o].kmer = kmer;
+          job[o].k = ik[o]; job[o].l = il[o]; job[o].c = ic[o]; job[o].n = &inn[o]; job[o].msg[0] = 0;
+          made[o] = (o+1 < S) && pthread_create(th+o,NULL,sort_worker,job+o) == 0;
+          if (!made[o])
+            sort_worker(job+o);
+        }
+      for (int o = 0; o < S; o++)
+        { if (made[o]) pthread_join(th[o],NULL);
+          if (job[o].rc != HM_OK && rc == HM_OK)
+            rc = hm_set_error(job[o].rc,"%s",job[o].msg);
+        }
+      s->launches += 6*S;
+    }
+  if (rc != HM_OK)
+    { for (int o = 0; o < S; o++)
+        { cudaSetDevice(s->d[o].dev); cudaFree(ik[o]); cudaFree(il[o]); cudaFree(ic[o]); }
+      if (raw_gone)
+        s->invalid = 1;                      /* the raw shards are gone */
+      return rc;
+    }
+  /* 5. the shards' new ranges, index and fingerprints */
+  int64_t pos = 0, nmax = 0;
+  for (int o = 0; o < S; o++)
+    { DevTable *O = s->d+o;
+      O->keys = ik[o]; O->keys_lo = il[o]; O->cnt = ic[o];
+      O->lo = pos; O->hi = pos+inn[o]; pos += inn[o];
+      if (inn[o] > nmax) nmax = inn[o];
+      s->cut[o] = cut[o];
+    }
+  s->n     = pos;
+  s->bits  = hm_pick_bucket_bits(s->n);
+  s->fpos  = hm_pick_filter_bits(s->n);
+  s->idx64 = (nmax >= 0xFFFFFFF0ll);
+  size_t ib = s->idx64 ? 8 : 4;
+  for (int o = 0; o < S && rc == HM_OK; o++)
+    { DevTable *O = s->d+o;
+      TRY(cudaSetDevice(O->dev));
+      dfree(O->dev,O->st,O->bucket); O->bucket = NULL;
+      TRY(cudaMalloc(&O->bucket,ib*(((size_t) 1<<s->bits)+1)));
+      TRY(cudaMemsetAsync(O->fp_acc,0,4*sizeof(uint64_t),O->st));
+      if (rc == HM_OK)
+        rc = hm_k_build_bucket_index(O->keys,O->hi-O->lo,s->bits,O->bucket,s->idx64,O->st);
+      if (rc == HM_OK)
+        rc = hm_k_symm_fingerprint(O->keys,O->keys_lo,O->cnt,0,O->hi-O->lo,kmer,s->seed,O->fp_acc,O->st);
+      s->launches += 2;
+    }
+  for (int o = 0; o < S; o++)
+    { cudaSetDevice(s->d[o].dev);
+      TRY(cudaStreamSynchronize(s->d[o].st));
+    }
+#undef TRY
+  if (rc == HM_OK)
+    rc = fingerprint_verdict(s);
+  if (rc != HM_OK)
+    { s->invalid = 1; return rc; }
+  s->aligned = 1;
+  return HM_OK;
+}
+
+extern "C" int hm_scan_shard_info(const hm_scan *s, int r, int *dev, int64_t *first_index, int64_t *n,
+                                  int64_t *device_bytes)
+{ if (s == NULL || r < 0 || r >= s->ngpu)
+    return hm_set_error(HM_EINVAL,"hm_scan_shard_info: no shard %d",r);
+  const DevTable *D = s->d+r;
+  int64_t na = s->sharded ? D->hi-D->lo : s->n;
+  if (dev)         *dev = D->dev;
+  if (first_index) *first_index = s->sharded ? D->lo : 0;
+  if (n)           *n = na;
+  if (device_bytes)
+    { int64_t b = (int64_t) sizeof(uint64_t)*(na+1)*(D->keys_lo ? 2 : 1) + (int64_t) sizeof(uint16_t)*(na+8)
+                + (s->idx64 ? 8 : 4)*(((int64_t) 1 << s->bits)+1) + (int64_t) sizeof(unsigned long long)*HM_PLOT_CELLS
+                + 4*(int64_t) sizeof(uint64_t);
+      if (D->symm_work != NULL) b += D->symm_layout.bytes;
+      *device_bytes = b;
+    }
   return HM_OK;
 }
 
@@ -567,10 +958,41 @@ static int ensure_direct(hm_scan *s)
   return rc;
 }
 
+/* sharded table: the key ranges are made run-aligned first (without conditioning, if that has not
+ * happened yet); shard r scans its own entries and fills Bloom segment r, segments sized for the
+ * largest shard; a key's owner is found by comparing it with the cuts                            */
+static int ensure_symm_sharded(hm_scan *s)
+{ int G = s->ngpu, rc;
+  if (!s->aligned && (rc = shard_partition(s,0,0,0)) != HM_OK)
+    return rc;
+  int64_t nmax = 1;
+  for (int g = 0; g < G; g++)
+    if (s->d[g].hi-s->d[g].lo > nmax) nmax = s->d[g].hi-s->d[g].lo;
+  for (int g = 0; g < G; g++)
+    { DevTable *D = s->d+g;
+      hm_symm_shards *sh = s->ssh+g;
+      memset(sh,0,sizeof(*sh));
+      sh->n_seg = G; sh->self = g;
+      for (int r = 0; r < G; r++)
+        { sh->off[r] = s->d[r].lo; sh->first_key[r] = r > 0 ? s->cut[r] : 0; }
+      sh->off[G] = s->n;
+      D->slo = 0; D->shi = D->hi-D->lo;
+      if ((rc = hm_symm_plan(nmax*G,D->shi,s->kmer,G,&D->symm_layout)) != HM_OK)
+        return rc;
+      HM_CUDA(cudaSetDevice(D->dev));
+      if (D->symm_work != NULL) { cudaFree(D->symm_work); D->symm_work = NULL; }
+      HM_CUDA(cudaMalloc(&D->symm_work,(size_t) D->symm_layout.bytes));
+    }
+  s->have_symm = 1;
+  return HM_OK;
+}
+
 /* work areas of the strand-symmetric scan (hm_symm.cu); several GPUs: cuts on run boundaries */
 static int ensure_symm(hm_scan *s)
 { if (s->have_symm)
     return HM_OK;
+  if (s->sharded)
+    return ensure_symm_sharded(s);
   int     G = s->ngpu;
   int64_t n = s->n, cut[HM_MAX_GPUS+1];
   cut[0] = 0; cut[G] = n;
@@ -614,6 +1036,18 @@ extern "C" int hm_scan_condition(hm_scan *s, int ethresh, int do_trim, int do_sy
   if (!do_trim && !do_symm)
     { if (nels_out) *nels_out = s->n;
       return HM_OK;
+    }
+  if (s->sharded)
+    { for (int g = 0; g < G; g++)
+        { DevTable *D = s->d+g;
+          HM_CUDA(cudaSetDevice(D->dev));
+          HM_CUDA(cudaStreamSynchronize(D->st));
+          if (D->symm_work != NULL) { cudaFree(D->symm_work); D->symm_work = NULL; }
+        }
+      s->have_symm = 0;
+      rc = shard_partition(s,ethresh,do_trim,do_symm);
+      if (nels_out) *nels_out = s->n;
+      return rc;
     }
   /* everything derived from the old table goes first: work buffers of both paths, the index */
   s->ran = 0; s->have_direct = 0; s->have_symm = 0;
@@ -687,80 +1121,87 @@ extern "C" int hm_scan_condition(hm_scan *s, int ethresh, int do_trim, int do_sy
   return rc != HM_OK ? rc : rc2;
 }
 
-/* reverse complement of a left-aligned packed k-mer (k <= 32) */
-static uint64_t revcomp64(uint64_t x, int k)
-{ x = ~x;
-  x = ((x >> 2)  & 0x3333333333333333ull) | ((x & 0x3333333333333333ull) << 2);
-  x = ((x >> 4)  & 0x0F0F0F0F0F0F0F0Full) | ((x & 0x0F0F0F0F0F0F0F0Full) << 4);
-  x = ((x >> 8)  & 0x00FF00FF00FF00FFull) | ((x & 0x00FF00FF00FF00FFull) << 8);
-  x = ((x >> 16) & 0x0000FFFF0000FFFFull) | ((x & 0x0000FFFF0000FFFFull) << 16);
-  x = (x >> 32) | (x << 32);
-  if (k < 32)
-    x = (x & (((uint64_t) 1 << (2*k))-1)) << (64-2*k);
-  return x;
-}
-
-/* reverse complement of a left-aligned packed k-mer of 33..64 bases held in two words */
-static void revcomp128(uint64_t hi, uint64_t lo, int k, uint64_t *rhi, uint64_t *rlo)
-{ /* reversing all 64 slots swaps the words; the k real bases end up right-aligned over 128 bits */
-  uint64_t a = revcomp64(lo,32), b = revcomp64(hi,32);      /* full-word reverse complements */
-  int      sh = 2*(64-k);                                    /* pad slots now sit on top: shift them out */
-  if (sh == 0) { *rhi = a; *rlo = b; }
-  else         { *rhi = (a << sh) | (b >> (64-sh)); *rlo = b << sh; }
-}
-
 /* examine_table (PloidyPlot.c:1167-1230).  trim: smallest non-zero count among the middle <=1e8
  * entries >= ethresh.  symm: reverse complement of entry 1 (moving on past palindromes, where
  * the reference's loop would never terminate) is present.                                      */
 extern "C" int hm_scan_examine(hm_scan *s, int ethresh, int *trim, int *symm)
-{ DevTable *D = s->d;
+{ /* the table as views: a replica is one view of the whole table on d[0]; a sharded table has one per
+   * shard, view v holding table indices [lo[v], hi[v]) at local index 0                              */
+  int       nv = s->sharded ? s->ngpu : 1;
+  int64_t   vlo[HM_MAX_GPUS], vhi[HM_MAX_GPUS];
   int64_t   n = s->n, frst, last;
   int       h_min = 0x8000, *d_min = NULL;
   uint64_t *d_q = NULL;
   int64_t  *d_pos = NULL;
-  int       two = (D->keys_lo != NULL);
+  int       two = (s->kmer > 32), rc = HM_OK;
+  if (s->invalid && s->sharded)
+    return hm_set_error(HM_EINVAL,"this scan was left unusable by a failed conditioning");
+  for (int v = 0; v < nv; v++)
+    { vlo[v] = s->sharded ? s->d[v].lo : 0; vhi[v] = s->sharded ? s->d[v].hi : n; }
 
-  HM_CUDA(cudaSetDevice(D->dev));
   if (n+3 < 100000000) { frst = 0; last = n; }
   else { frst = n/2-50000000; last = n/2+50000000; }
-  HM_CUDA(cudaMalloc(&d_min,sizeof(int)));
-  HM_CUDA(cudaMemcpyAsync(d_min,&h_min,sizeof(int),cudaMemcpyHostToDevice,D->st));
-  int rc = hm_k_min_count(D->cnt,frst,last,d_min,D->st);
-  s->launches += 1;
-  if (rc == HM_OK)
-    { cudaError_t e = cudaMemcpyAsync(&h_min,d_min,sizeof(int),cudaMemcpyDeviceToHost,D->st);
-      if (e == cudaSuccess) e = cudaStreamSynchronize(D->st);
-      if (e != cudaSuccess) rc = hm_cuda_fail(e,"min_count");
+  for (int v = 0; v < nv && rc == HM_OK; v++)            /* min over the middle entries = min of the views' minima */
+    { DevTable *D = s->d+v;
+      int64_t   a = frst > vlo[v] ? frst : vlo[v], b = last < vhi[v] ? last : vhi[v];
+      int       vmin = 0x8000;
+      if (a >= b) continue;
+      HM_CUDA(cudaSetDevice(D->dev));
+      HM_CUDA(cudaMalloc(&d_min,sizeof(int)));
+      HM_CUDA(cudaMemcpyAsync(d_min,&vmin,sizeof(int),cudaMemcpyHostToDevice,D->st));
+      rc = hm_k_min_count(D->cnt,a-vlo[v],b-vlo[v],d_min,D->st);
+      s->launches += 1;
+      if (rc == HM_OK)
+        { cudaError_t e = cudaMemcpyAsync(&vmin,d_min,sizeof(int),cudaMemcpyDeviceToHost,D->st);
+          if (e == cudaSuccess) e = cudaStreamSynchronize(D->st);
+          if (e != cudaSuccess) rc = hm_cuda_fail(e,"min_count");
+        }
+      cudaFree(d_min);
+      if (vmin < h_min) h_min = vmin;
     }
-  cudaFree(d_min);
   if (rc != HM_OK)
     return rc;
   *trim = (h_min >= ethresh);
 
+  /* entry sidx from the view that holds it, its reverse complement looked up by key (in whichever
+   * view has it: the key ranges of the views do not overlap)                                    */
   *symm = 1;
-  HM_CUDA(cudaMalloc(&d_q,2*sizeof(uint64_t)));
-  HM_CUDA(cudaMalloc(&d_pos,sizeof(int64_t)));
-  for (int64_t sidx = 1; sidx < n; sidx++)
+  for (int64_t sidx = 1; sidx < n && rc == HM_OK; sidx++)
     { uint64_t x, xw = 0, q[2];
-      int64_t  pos;
-      cudaError_t e = cudaMemcpyAsync(&x,D->keys+sidx,sizeof(uint64_t),cudaMemcpyDeviceToHost,D->st);
+      int64_t  pos = -1;
+      int      u = 0;
+      while (u+1 < nv && sidx >= vhi[u]) u++;
+      DevTable *D = s->d+u;
+      HM_CUDA(cudaSetDevice(D->dev));
+      cudaError_t e = cudaMemcpyAsync(&x,D->keys+(sidx-vlo[u]),sizeof(uint64_t),cudaMemcpyDeviceToHost,D->st);
       if (e == cudaSuccess && two)
-        e = cudaMemcpyAsync(&xw,D->keys_lo+sidx,sizeof(uint64_t),cudaMemcpyDeviceToHost,D->st);
+        e = cudaMemcpyAsync(&xw,D->keys_lo+(sidx-vlo[u]),sizeof(uint64_t),cudaMemcpyDeviceToHost,D->st);
       if (e == cudaSuccess) e = cudaStreamSynchronize(D->st);
       if (e != cudaSuccess) { rc = hm_cuda_fail(e,"examine: key fetch"); break; }
       if (two) revcomp128(x,xw,s->kmer,q,q+1);
       else     { q[0] = revcomp64(x,s->kmer); q[1] = 0; }
-      cudaMemcpyAsync(d_q,q,2*sizeof(uint64_t),cudaMemcpyHostToDevice,D->st);
-      rc = hm_k_find_keys(D->keys,D->keys_lo,n,D->bucket,s->bits,s->idx64,d_q,two ? d_q+1 : NULL,1,d_pos,D->st);
-      s->launches += 1;
+      for (int v = 0; v < nv && rc == HM_OK && pos < 0; v++)
+        { DevTable *V = s->d+v;
+          int64_t   p = -1;
+          if (vhi[v] <= vlo[v]) continue;
+          HM_CUDA(cudaSetDevice(V->dev));
+          HM_CUDA(cudaMalloc(&d_q,2*sizeof(uint64_t)));
+          HM_CUDA(cudaMalloc(&d_pos,sizeof(int64_t)));
+          cudaMemcpyAsync(d_q,q,2*sizeof(uint64_t),cudaMemcpyHostToDevice,V->st);
+          rc = hm_k_find_keys(V->keys,V->keys_lo,vhi[v]-vlo[v],V->bucket,s->bits,s->idx64,d_q,two ? d_q+1 : NULL,1,d_pos,V->st);
+          s->launches += 1;
+          if (rc == HM_OK)
+            { e = cudaMemcpyAsync(&p,d_pos,sizeof(int64_t),cudaMemcpyDeviceToHost,V->st);
+              if (e == cudaSuccess) e = cudaStreamSynchronize(V->st);
+              if (e != cudaSuccess) rc = hm_cuda_fail(e,"examine: lookup");
+            }
+          cudaFree(d_q); cudaFree(d_pos);
+          if (p >= 0) pos = vlo[v]+p;
+        }
       if (rc != HM_OK) break;
-      e = cudaMemcpyAsync(&pos,d_pos,sizeof(int64_t),cudaMemcpyDeviceToHost,D->st);
-      if (e == cudaSuccess) e = cudaStreamSynchronize(D->st);
-      if (e != cudaSuccess) { rc = hm_cuda_fail(e,"examine: lookup"); break; }
       if (pos < 0) { *symm = 0; break; }
       if (pos != sidx) { *symm = 1; break; }
     }
-  cudaFree(d_q); cudaFree(d_pos);
   return rc;
 }
 
@@ -901,6 +1342,12 @@ static int run_symm(hm_scan *s, int64_t *plot, hm_scan_stats *stats, uint64_t *s
   float       ms1 = 0, ms2 = 0, msall = 0;
   if ((rc = ensure_symm(s)) != HM_OK)
     return rc;
+  hm_shard_tabs tabs;                           /* sharded: pass 2 settles Bloom hits in the owner's arrays */
+  memset(&tabs,0,sizeof(tabs));
+  for (int g = 0; g < G && s->sharded; g++)
+    { tabs.keys[g] = s->d[g].keys; tabs.keys_lo[g] = s->d[g].keys_lo; tabs.cnt[g] = s->d[g].cnt;
+      tabs.bucket[g] = s->d[g].bucket; tabs.n[g] = s->d[g].hi-s->d[g].lo;
+    }
   double      t0 = now_ms();
   for (int g = 0; g < G; g++)
     { DevTable *D = s->d+g;
@@ -909,10 +1356,11 @@ static int run_symm(hm_scan *s, int64_t *plot, hm_scan_stats *stats, uint64_t *s
         HM_CUDA(cudaEventCreate(&ev[g][k]));
       HM_CUDA(cudaEventRecord(ev[g][0],D->st));
       HM_CUDA(cudaMemsetAsync(D->plot,0,sizeof(unsigned long long)*HM_PLOT_CELLS,D->st));
-      rc = hm_k_symm_runscan(D->keys,D->keys_lo,D->cnt,n,D->bucket,s->bits,s->idx64,s->kmer,D->slo,D->shi,
+      int64_t na = s->sharded ? D->hi-D->lo : n;         /* entries in this device's arrays */
+      rc = hm_k_symm_runscan(D->keys,D->keys_lo,D->cnt,na,D->bucket,s->bits,s->idx64,s->kmer,D->slo,D->shi,
                              D->symm_work,&D->symm_layout,G > 1 ? &s->ssh[g] : NULL,D->st);
       if (rc == HM_OK)
-        rc = hm_k_symm_runs(D->keys,D->keys_lo,D->cnt,n,D->bucket,s->bits,s->idx64,s->kmer,D->slo,D->shi,
+        rc = hm_k_symm_runs(D->keys,D->keys_lo,D->cnt,na,D->bucket,s->bits,s->idx64,s->kmer,D->slo,D->shi,
                             D->symm_work,&D->symm_layout,G > 1 ? &s->ssh[g] : NULL,D->st);
       if (rc != HM_OK) return rc;
       s->launches += 2*(D->shi > D->slo);
@@ -938,8 +1386,12 @@ static int run_symm(hm_scan *s, int64_t *plot, hm_scan_stats *stats, uint64_t *s
     { DevTable *D = s->d+g;
       HM_CUDA(cudaSetDevice(D->dev));
       HM_CUDA(cudaEventRecord(ev[g][2],D->st));
-      rc = hm_k_symm_resolve(D->keys,D->keys_lo,D->cnt,n,D->bucket,s->bits,s->idx64,s->kmer,
-                             D->symm_work,&D->symm_layout,G > 1 ? &s->ssh[g] : NULL,D->plot,D->st);
+      if (s->sharded)
+        rc = hm_symm_resolve_sharded(&tabs,s->bits,s->idx64,s->kmer,D->symm_work,&D->symm_layout,
+                                     G > 1 ? &s->ssh[g] : NULL,D->plot,D->st);
+      else
+        rc = hm_k_symm_resolve(D->keys,D->keys_lo,D->cnt,n,D->bucket,s->bits,s->idx64,s->kmer,
+                               D->symm_work,&D->symm_layout,G > 1 ? &s->ssh[g] : NULL,D->plot,D->st);
       if (rc != HM_OK) return rc;
       s->launches += 1;
       HM_CUDA(cudaEventRecord(ev[g][3],D->st));
@@ -1000,6 +1452,26 @@ extern "C" int hm_scan_is_symmetric(const hm_scan *s) { return s->symmetric; }
 extern "C" int hm_scan_run_path(hm_scan *s, int path, int64_t *plot, hm_scan_stats *stats)
 { if (s->invalid)
     return hm_set_error(HM_EINVAL,"this scan was left unusable by a failed conditioning");
+  if (s->sharded)
+    { if (path == HM_PATH_DIRECT)
+        return hm_set_error(HM_EUNSUPPORTED,"a sharded table has only the strand-symmetric scan (the direct "
+                                            "passes need the whole table on every GPU)");
+      if (path != HM_PATH_AUTO && path != HM_PATH_SYMM)
+        return hm_set_error(HM_EINVAL,"hm_scan_run_path: unknown path %d",path);
+      int rc;
+      if (!s->aligned && (rc = ensure_symm(s)) != HM_OK)     /* the verdict is taken on the aligned shards */
+        return rc;
+      if (!s->symmetric)
+        return hm_set_error(HM_EUNSUPPORTED,"the table is not strand-symmetric: a sharded table can only be "
+                                            "scanned after conditioning (hm_scan_condition)");
+      uint64_t status = 0;
+      if ((rc = run_symm(s,plot,stats,&status)) != HM_OK)
+        return rc;
+      if (status != 0)
+        return hm_set_error(HM_EUNSUPPORTED,"symmetric scan of a sharded table failed its own checks (status %llu); "
+                                            "the direct passes cannot stand in for it",(unsigned long long) status);
+      return HM_OK;
+    }
   if (path == HM_PATH_AUTO)
     { const char *e = getenv("HETMERS_PATH");
       if (e != NULL && strcmp(e,"direct") == 0) path = HM_PATH_DIRECT;
@@ -1056,6 +1528,8 @@ extern "C" int hm_scan_extract(hm_scan *s, const uint16_t *pixmap, hm_pair_rec *
 { int G = s->ngpu, rc = HM_OK;
   if (s->invalid)
     return hm_set_error(HM_EINVAL,"this scan was left unusable by a failed conditioning");
+  if (s->sharded)
+    return hm_set_error(HM_EUNSUPPORTED,"extract_kmer_pairs needs the direct passes, which a sharded table does not have");
   if ((rc = need_direct_results(s)) != HM_OK)
     return rc;
   int64_t      total = 0, cnts[HM_MAX_GPUS];
@@ -1121,7 +1595,25 @@ extern "C" int hm_hetmers_host(const hm_host_table *t, const int *dev, int n_gpu
 }
 
 extern "C" int hm_scan_download(hm_scan *s, uint64_t *keys, uint64_t *keys_lo, uint16_t *cnt, uint8_t *deg)
-{ DevTable *D = s->d;
+{ if (s->sharded)                       /* the concatenation of the shards */
+    { if (deg != NULL)
+        return hm_set_error(HM_EUNSUPPORTED,"a sharded table has no incidence array (pass deg = NULL)");
+      if (s->invalid)
+        return hm_set_error(HM_EINVAL,"this scan was left unusable by a failed conditioning");
+      for (int g = 0; g < s->ngpu; g++)
+        { DevTable *O = s->d+g;
+          size_t    m = (size_t) (O->hi-O->lo);
+          if (m == 0) continue;
+          HM_CUDA(cudaSetDevice(O->dev));
+          HM_CUDA(cudaStreamSynchronize(O->st));
+          if (keys != NULL)    HM_CUDA(cudaMemcpy(keys+O->lo,O->keys,sizeof(uint64_t)*m,cudaMemcpyDeviceToHost));
+          if (keys_lo != NULL && O->keys_lo != NULL)
+                               HM_CUDA(cudaMemcpy(keys_lo+O->lo,O->keys_lo,sizeof(uint64_t)*m,cudaMemcpyDeviceToHost));
+          if (cnt != NULL)     HM_CUDA(cudaMemcpy(cnt+O->lo,O->cnt,sizeof(uint16_t)*m,cudaMemcpyDeviceToHost));
+        }
+      return HM_OK;
+    }
+  DevTable *D = s->d;
   HM_CUDA(cudaSetDevice(D->dev));
   HM_CUDA(cudaStreamSynchronize(D->st));
   if (keys != NULL)

@@ -43,6 +43,7 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <type_traits>
 
 #include "hetmers_b200.h"
 #include "hm_internal.h"
@@ -1187,13 +1188,32 @@ __device__ __noinline__ bool has_upper_partner(const uint64_t *__restrict__ keys
   return (U > 0);
 }
 
+/* per-shard tables of a sharded scan (every shard holds only its own key range, DESIGN.md §6): the exact
+ * check of a Bloom hit reads rc x's run in the arrays of the shard that owns it, as peer memory       */
+typedef hm_shard_tabs ShardTabs;
+struct NoTabs {};                                           /* a replica: the table is local */
+
+template <typename IdxT, int KW, typename Tabs>
+__device__ __forceinline__ bool exact_upper_partner(const uint64_t *__restrict__ keys, const uint64_t *__restrict__ keys_lo,
+                                                    const uint16_t *__restrict__ cnt, int64_t n,
+                                                    const IdxT *__restrict__ bucket, int bshift, int kmer,
+                                                    const SymmView &W, const Tabs &T, uint64_t q, uint64_t ql, int cq)
+{ if constexpr (std::is_same<Tabs,ShardTabs>::value)
+    { const int o = W.n_seg > 1 ? owner_of(W,q) : 0;
+      return has_upper_partner<IdxT,KW>(T.keys[o],T.keys_lo[o],T.cnt[o],T.n[o],(const IdxT *) T.bucket[o],
+                                        bshift,kmer,q,ql,cq,W.status);
+    }
+  else
+    return has_upper_partner<IdxT,KW>(keys,keys_lo,cnt,n,bucket,bshift,kmer,q,ql,cq,W.status);
+}
+
 /* one candidate: are rc x / rc y in S?  Bloom bits first; EXACT = also settle the hits.
  * -> 0 isolated pair, 1 not isolated, 2 undecided (a Bloom hit, EXACT == false)                  */
-template <typename IdxT, int KW, bool EXACT>
+template <typename IdxT, int KW, bool EXACT, typename Tabs>
 __device__ __forceinline__ int judge_candidate(const uint64_t *__restrict__ keys, const uint64_t *__restrict__ keys_lo,
                                                const uint16_t *__restrict__ cnt, int64_t n,
                                                const IdxT *__restrict__ bucket, int bshift, int kmer,
-                                               const SymmView &W, uint64_t x, uint64_t xl, uint64_t meta)
+                                               const SymmView &W, const Tabs &T, uint64_t x, uint64_t xl, uint64_t meta)
 { const int cx = (int) (meta & 0xffff), cy = (int) ((meta >> 16) & 0xffff);
   const int p  = (int) ((meta >> 32) & 0xff), yb = (int) ((meta >> 40) & 3);
   uint64_t rx, rxl, ry, ryl;
@@ -1210,9 +1230,9 @@ __device__ __forceinline__ int judge_candidate(const uint64_t *__restrict__ keys
     return 0;
   if (!EXACT)
     return 2;
-  if (ha && has_upper_partner<IdxT,KW>(keys,keys_lo,cnt,n,bucket,bshift,kmer,rx,rxl,cx,W.status))
+  if (ha && exact_upper_partner<IdxT,KW>(keys,keys_lo,cnt,n,bucket,bshift,kmer,W,T,rx,rxl,cx))
     return 1;
-  if (hb && has_upper_partner<IdxT,KW>(keys,keys_lo,cnt,n,bucket,bshift,kmer,ry,ryl,cy,W.status))
+  if (hb && exact_upper_partner<IdxT,KW>(keys,keys_lo,cnt,n,bucket,bshift,kmer,W,T,ry,ryl,cy))
     return 1;
   return 0;
 }
@@ -1235,11 +1255,11 @@ __device__ __forceinline__ void count_pair(uint32_t *tile, unsigned long long *_
  * lane does that stalls all 32: they are parked in a per-warp queue and settled 32 at a time, every
  * lane busy.  RV_ILP candidates per thread and trip keep that many record / Bloom loads in flight
  * (the kernel is bound by the latency of record -> Bloom word, not by bytes or instructions).         */
-template <typename IdxT, int KW>
-__global__ void __launch_bounds__(RV_THREADS,RV_CTAS_PER_SM)
-resolve_kernel(const uint64_t *__restrict__ keys, const uint64_t *__restrict__ keys_lo,
-               const uint16_t *__restrict__ cnt, int64_t n, const IdxT *__restrict__ bucket, int bshift,
-               int kmer, const SymmView W, unsigned long long *__restrict__ plot)
+template <typename IdxT, int KW, typename Tabs>
+__device__ __forceinline__ void resolve_body(const uint64_t *__restrict__ keys, const uint64_t *__restrict__ keys_lo,
+                                             const uint16_t *__restrict__ cnt, int64_t n, const IdxT *__restrict__ bucket,
+                                             int bshift, int kmer, const SymmView &W, const Tabs &T,
+                                             unsigned long long *__restrict__ plot)
 { extern __shared__ uint32_t tile[];
   __shared__ uint32_t s_q[RV_THREADS/32][32*(RV_ILP+1)];
   const unsigned FULL = 0xffffffffu;
@@ -1305,7 +1325,7 @@ resolve_kernel(const uint64_t *__restrict__ keys, const uint64_t *__restrict__ k
           __syncwarp();
           const int64_t j = first-lane + (int64_t) (e & 31) + (int64_t) (e >> 5)*stride;
           const uint64_t xx = W.cand_key[j], xxl = KW == 2 ? W.cand_lo[j] : 0, mm = W.cand_meta[j];
-          if (judge_candidate<IdxT,KW,true>(keys,keys_lo,cnt,n,bucket,bshift,kmer,W,xx,xxl,mm) == 0)
+          if (judge_candidate<IdxT,KW,true>(keys,keys_lo,cnt,n,bucket,bshift,kmer,W,T,xx,xxl,mm) == 0)
             count_pair(tile,plot,mm,kmer);
         }
     }
@@ -1313,7 +1333,7 @@ resolve_kernel(const uint64_t *__restrict__ keys, const uint64_t *__restrict__ k
     { const uint32_t e = q[lane];
       const int64_t j = first-lane + (int64_t) (e & 31) + (int64_t) (e >> 5)*stride;
       const uint64_t xx = W.cand_key[j], xxl = KW == 2 ? W.cand_lo[j] : 0, mm = W.cand_meta[j];
-      if (judge_candidate<IdxT,KW,true>(keys,keys_lo,cnt,n,bucket,bshift,kmer,W,xx,xxl,mm) == 0)
+      if (judge_candidate<IdxT,KW,true>(keys,keys_lo,cnt,n,bucket,bshift,kmer,W,T,xx,xxl,mm) == 0)
         count_pair(tile,plot,mm,kmer);
     }
   __syncthreads();
@@ -1322,6 +1342,21 @@ resolve_kernel(const uint64_t *__restrict__ keys, const uint64_t *__restrict__ k
       if (v != 0)
         atomicAdd(plot + (t/RV_TM)*HM_PLOT_W + (t%RV_TM), (unsigned long long) v);
     }
+}
+
+template <typename IdxT, int KW>
+__global__ void __launch_bounds__(RV_THREADS,RV_CTAS_PER_SM)
+resolve_kernel(const uint64_t *__restrict__ keys, const uint64_t *__restrict__ keys_lo,
+               const uint16_t *__restrict__ cnt, int64_t n, const IdxT *__restrict__ bucket, int bshift,
+               int kmer, const SymmView W, unsigned long long *__restrict__ plot)
+{ resolve_body<IdxT,KW>(keys,keys_lo,cnt,n,bucket,bshift,kmer,W,NoTabs(),plot); }
+
+/* pass 2 of a sharded scan: the same, with every Bloom hit settled in the owner's arrays */
+template <typename IdxT, int KW>
+__global__ void __launch_bounds__(RV_THREADS,RV_CTAS_PER_SM)
+resolve_sharded_kernel(int bshift, int kmer, const SymmView W, const ShardTabs T, unsigned long long *__restrict__ plot)
+{ resolve_body<IdxT,KW>((const uint64_t *) NULL,(const uint64_t *) NULL,(const uint16_t *) NULL,(int64_t) 0,
+                        (const IdxT *) NULL,bshift,kmer,W,T,plot);
 }
 
 template <typename IdxT, int KW>
@@ -1367,6 +1402,47 @@ extern "C" int hm_k_symm_resolve(const uint64_t *d_keys, const uint64_t *d_keys_
     bloom_window(st,NULL,0,0);
   if (e != cudaSuccess)
     return hm_cuda_fail(e,"resolve_kernel");
+  return HM_OK;
+}
+
+template <typename IdxT, int KW>
+static cudaError_t launch_resolve_sharded(int bits, int kmer, const SymmView &W, const ShardTabs &T,
+                                          unsigned long long *plot, int64_t range, cudaStream_t st)
+{ static int configured[64] = {0};
+  size_t smem = (size_t) RV_TS*RV_TM*sizeof(uint32_t);
+  int dev = 0, sms = 148;
+  cudaGetDevice(&dev);
+  if (dev >= 64 || !configured[dev])
+    { cudaError_t e = cudaFuncSetAttribute(resolve_sharded_kernel<IdxT,KW>,cudaFuncAttributeMaxDynamicSharedMemorySize,(int) smem);
+      if (e != cudaSuccess) return e;
+      if (dev < 64) configured[dev] = 1;
+    }
+  cudaDeviceGetAttribute(&sms,cudaDevAttrMultiProcessorCount,dev);
+  int64_t want = (range/8+RV_THREADS-1)/RV_THREADS;
+  int     grid = (int) (want < sms*RV_CTAS_PER_SM ? (want > 0 ? want : 1) : sms*RV_CTAS_PER_SM);
+  resolve_sharded_kernel<IdxT,KW><<<grid,RV_THREADS,smem,st>>>(64-bits,kmer,W,T,plot);
+  return cudaGetLastError();
+}
+
+/* pass 2 of a sharded table: tabs holds every shard's arrays as addressable from the calling device */
+int hm_symm_resolve_sharded(const hm_shard_tabs *tabs, int bits, int idx64, int kmer, void *d_work,
+                            const hm_symm_layout *layout, const hm_symm_shards *shards,
+                            unsigned long long *d_plot, void *stream)
+{ if (kmer < HM_SYMM_MIN_KMER || kmer > HM_MAX_KMER || tabs == NULL || d_work == NULL || layout == NULL || d_plot == NULL)
+    return hm_set_error(HM_EINVAL,"symm_resolve_sharded: bad arguments");
+  cudaStream_t st = (cudaStream_t) stream;
+  SymmView W = make_view(d_work,layout,shards);
+  cudaError_t e;
+  if (kmer <= 32)
+    e = idx64 ? launch_resolve_sharded<uint64_t,1>(bits,kmer,W,*tabs,d_plot,layout->range,st)
+              : launch_resolve_sharded<uint32_t,1>(bits,kmer,W,*tabs,d_plot,layout->range,st);
+  else
+    e = idx64 ? launch_resolve_sharded<uint64_t,2>(bits,kmer,W,*tabs,d_plot,layout->range,st)
+              : launch_resolve_sharded<uint32_t,2>(bits,kmer,W,*tabs,d_plot,layout->range,st);
+  if (l2_persist())
+    bloom_window(st,NULL,0,0);
+  if (e != cudaSuccess)
+    return hm_cuda_fail(e,"resolve_sharded_kernel");
   return HM_OK;
 }
 

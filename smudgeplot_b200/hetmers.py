@@ -100,18 +100,33 @@ def _host_table(kt: KtabFiles):
 
 
 class Scan:
-    """Device-resident table + both passes (hm_scan_*)."""
+    """Device-resident table + both passes (hm_scan_*).  shards=[d0, d1, ...]: sharded placement, shard r
+    on device d_r (a device may carry several shards): each holds only its own key range, so the table
+    may exceed one GPU's memory; only the strand-symmetric scan runs on such a table."""
 
-    def __init__(self, kt: KtabFiles, gpus: int = 1, devices=None):
+    def __init__(self, kt: KtabFiles, gpus: int = 1, devices=None, shards=None):
         L = _lib.lib()
         self._L = L
+        self._h = None
         self.kt = kt
         ht, self._keep = _host_table(kt)
-        devs = list(devices) if devices is not None else list(range(gpus))
+        self.sharded = shards is not None
+        devs = list(shards) if shards is not None else (list(devices) if devices is not None else list(range(gpus)))
         arr = (C.c_int * len(devs))(*devs)
         h = C.c_void_p()
-        _lib.check(L.hm_scan_create(C.byref(ht), arr, len(devs), C.byref(h)))
+        create = L.hm_scan_create_sharded if self.sharded else L.hm_scan_create
+        _lib.check(create(C.byref(ht), arr, len(devs), C.byref(h)))
         self._h = h
+        self.n_dev = len(devs)
+
+    def shard_info(self):
+        """per shard (or replica): dict(dev, first_index, n, device_bytes) -- hm_scan_shard_info"""
+        out = []
+        for r in range(self.n_dev):
+            d, f, n, b = C.c_int(), C.c_int64(), C.c_int64(), C.c_int64()
+            _lib.check(self._L.hm_scan_shard_info(self._h, r, C.byref(d), C.byref(f), C.byref(n), C.byref(b)))
+            out.append({"dev": d.value, "first_index": f.value, "n": n.value, "device_bytes": b.value})
+        return out
 
     def examine(self, ethresh: int):
         """(trimmed?, symmetric?) as examine_table decides them (PloidyPlot.c:1167-1230)."""
@@ -160,7 +175,13 @@ class Scan:
         return arr
 
     def download(self, deg: bool = True):
-        n = getattr(self, "nels", self.kt.nels)
+        """-> (keys, cnt, deg) of the device table; a sharded table gives the concatenation of its shards
+        (run a scan or condition() first: that fixes the shards' key ranges) and no deg"""
+        if self.sharded:
+            deg = False
+            n = sum(s["n"] for s in self.shard_info())
+        else:
+            n = getattr(self, "nels", self.kt.nels)
         keys = np.empty(n, dtype=np.uint64)
         klo = np.empty(n, dtype=np.uint64) if self.kt.kmer > 32 else None
         cnt = np.empty(n, dtype=np.uint16)

@@ -233,6 +233,32 @@ static int pick_gpus(int *devs)
   return (ngpu);
 }
 
+/* Placement of the table on the ngpu devices (hm_plan_placement, from what each device has free):
+ * a full replica on every GPU whenever one fits, else one shard per GPU, else neither.           */
+static int plan_placement(const hm_host_table *t, const int *devs, int ngpu, int do_symm, hm_scan *held)
+{ int64_t fr[16];
+  for (int g = 0; g < ngpu; g++)
+    { if (hm_device_free_bytes(devs[g],&fr[g]) != HM_OK)
+        die_hm();
+      if (held != NULL)               /* what the loaded table takes is free again if it is re-placed */
+        { int64_t b = 0;
+          if (hm_scan_shard_info(held,g,NULL,NULL,NULL,&b) != HM_OK)
+            die_hm();
+          fr[g] += b;
+        }
+    }
+  int r = hm_plan_placement(t->kmer,t->nels,do_symm,ngpu,fr,NULL,NULL);
+  if (r < 0)
+    die_hm();
+  return r;
+}
+
+static void does_not_fit(const hm_host_table *t, int ngpu)
+{ fprintf(stderr,"%s: a table of %lld k-mers does not fit on %d GPUs, not even sharded over them; "
+                 "set HETMERS_GPUS to use more GPUs\n",Prog_Name,(long long) t->nels,ngpu);
+  exit (1);
+}
+
 int main(int argc, char *argv[])
 { int    VERBOSE = 0, NTHREADS = 4, ETHRESH = 4;
   const char *SORT_PATH = "/tmp";
@@ -352,7 +378,7 @@ int main(int argc, char *argv[])
   hm_table *T;
   hm_scan  *S;
   char     *input = NULL;
-  int       ngpu, devs[16];
+  int       ngpu, devs[16], place = HM_PLACE_REPLICA;
   double    t_start = wall_ms(), t_open, t_load, t_exam, t_scan;
 
   start_cuda_early();            /* background: nothing below waits for it before hm_device_count() */
@@ -379,7 +405,14 @@ int main(int argc, char *argv[])
       { fprintf(stderr,"%s: k-mer table %s has fewer than 2 entries\n",Prog_Name,SRC);
         exit (1);
       }
-    if (hm_scan_create(hm_table_view(T),devs,ngpu,&S) != HM_OK)
+    place = plan_placement(hm_table_view(T),devs,ngpu,0,NULL);
+    if (place == HM_PLACE_NOFIT && ngpu > 1)
+      does_not_fit(hm_table_view(T),ngpu);
+    if (place == HM_PLACE_SHARDED)
+      { if (hm_scan_create_sharded(hm_table_view(T),devs,ngpu,&S) != HM_OK)
+          die_hm();
+      }
+    else if (hm_scan_create(hm_table_view(T),devs,ngpu,&S) != HM_OK)
       die_hm();
     t_load = wall_ms();
     if (hm_scan_examine(S,ETHRESH,&trim,&symm) != HM_OK)
@@ -412,6 +445,17 @@ int main(int argc, char *argv[])
         int64_t nn;
         if (!trim) announce_step(VERBOSE,'t',trim,ETHRESH);
         if (!symm) announce_step(VERBOSE,'s',trim,ETHRESH);
+        if (!symm)                      /* symmetrising doubles the table: placed again for that */
+          { int p2 = plan_placement(hm_table_view(T),devs,ngpu,1,S);
+            if (p2 == HM_PLACE_NOFIT && ngpu > 1)
+              does_not_fit(hm_table_view(T),ngpu);
+            if (p2 == HM_PLACE_SHARDED && place == HM_PLACE_REPLICA)
+              { hm_scan_destroy(S);
+                place = HM_PLACE_SHARDED;
+                if (hm_scan_create_sharded(hm_table_view(T),devs,ngpu,&S) != HM_OK)
+                  die_hm();
+              }
+          }
         if (hm_scan_condition(S,ETHRESH,!trim,!symm,&nn) != HM_OK)
           die_hm();
         if (nn < 2)
@@ -453,7 +497,12 @@ int main(int argc, char *argv[])
           { fprintf(stderr,"%s: Cannot open k-mer table %s\n",Prog_Name,input);
             exit (1);
           }
-        if (hm_scan_create(hm_table_view(T),devs,ngpu,&S) != HM_OK)
+        place = plan_placement(hm_table_view(T),devs,ngpu,0,NULL);
+        if (place == HM_PLACE_SHARDED)
+          { if (hm_scan_create_sharded(hm_table_view(T),devs,ngpu,&S) != HM_OK)
+              die_hm();
+          }
+        else if (hm_scan_create(hm_table_view(T),devs,ngpu,&S) != HM_OK)
           die_hm();
       }
   }
@@ -483,7 +532,16 @@ int main(int argc, char *argv[])
   //   context by hand costs ~0.1 s of wall clock for nothing)
 
   if (getenv("HETMERS_STATS") != NULL)
-    fprintf(stderr,"{\"nels\": %lld, \"n_gpus\": %d, \"path\": \"%s\", \"bucket_bits\": %d, \"ms_load\": %.3f, "
+    { fprintf(stderr,"{\"placement\": \"%s\", \"device_bytes\": [",place == HM_PLACE_SHARDED ? "sharded" : "replica");
+      for (i = 0; i < ngpu; i++)
+        { int64_t b = 0;
+          hm_scan_shard_info(S,i,NULL,NULL,NULL,&b);
+          fprintf(stderr,"%s%lld",i ? ", " : "",(long long) b);
+        }
+      fprintf(stderr,"], ");
+    }
+  if (getenv("HETMERS_STATS") != NULL)
+    fprintf(stderr,"\"nels\": %lld, \"n_gpus\": %d, \"path\": \"%s\", \"bucket_bits\": %d, \"ms_load\": %.3f, "
                    "\"ms_pass1\": %.3f, \"ms_pass2\": %.3f, \"ms_scan\": %.3f, \"kernel_launches\": %lld, "
                    "\"wall_ms\": {\"open\": %.1f, \"cuda_init_load\": %.1f, \"examine\": %.1f, \"scan\": %.1f}, "
                    "\"load_ms\": {\"alloc\": %.1f, \"records\": %.1f, \"index\": %.1f}}\n",
