@@ -296,6 +296,21 @@ int  hm_scan_is_symmetric(const hm_scan *s);
 /* the pair list of extract_kmer_pairs (runs the direct passes first if the last run did not) for a pixel->smudge map (host
  * uint16[HM_PLOT_CELLS]); *out is malloc'ed (caller frees), sorted by (smudge, k-mer).          */
 int  hm_scan_extract(hm_scan *s, const uint16_t *pixmap, hm_pair_rec **out, int64_t *n_out);
+/* the same list by either route.  HM_PATH_SYMM judges the candidates the symmetric scan left on the
+ * devices again and writes the records of the isolated, labelled ones (running that scan first if
+ * there was none since the last conditioning, or it fell back to the direct passes); it works on
+ * sharded tables, allocates no device memory and is HM_EINVAL on a table that is not strand-symmetric
+ * or has k < HM_SYMM_MIN_KMER.  HM_PATH_DIRECT is hm_scan_extract.  HM_PATH_AUTO takes the path
+ * hm_scan_run takes (HETMERS_PATH included).  stats (may be NULL): the path taken, the number of
+ * slices the candidates were judged in, the records, and the times of the extraction kernels, of
+ * copying the records to the host and of sorting them there.                                      */
+typedef struct hm_extract_stats
+  { int32_t path, slices;
+    int64_t n_records;
+    double  ms_kernel, ms_copy, ms_sort;
+  } hm_extract_stats;
+int  hm_scan_extract_path(hm_scan *s, int path, const uint16_t *pixmap, hm_pair_rec **out, int64_t *n_out,
+                          hm_extract_stats *stats);
 /* one call: create + run + destroy (what bench.py's e2e leg times) */
 int  hm_hetmers_host(const hm_host_table *t, const int *dev, int n_gpus,
                      int64_t *plot, hm_scan_stats *stats);
@@ -309,8 +324,9 @@ int  hm_scan_download(hm_scan *s, uint64_t *keys, uint64_t *keys_lo, uint16_t *c
  * may carry several logical shards.  Each shard loads 1/n_shards of the part files; the key ranges
  * are established by the first hm_scan_condition (which trims / symmetrises on the way) or, for a
  * table that needs no conditioning, by the first scan.  On a sharded scan hm_scan_examine,
- * hm_scan_condition, hm_scan_run / hm_scan_run_path(HM_PATH_SYMM) and hm_scan_download work;
- * hm_scan_extract, HM_PATH_DIRECT and tables that are not strand-symmetric are HM_EUNSUPPORTED.    */
+ * hm_scan_condition, hm_scan_run / hm_scan_run_path(HM_PATH_SYMM), hm_scan_extract_path (HM_PATH_AUTO /
+ * HM_PATH_SYMM) and hm_scan_download work; hm_scan_extract, HM_PATH_DIRECT and tables that are not
+ * strand-symmetric are HM_EUNSUPPORTED.                                                             */
 int  hm_scan_create_sharded(const hm_host_table *t, const int *dev, int n_shards, hm_scan **out);
 /* shard r: device, index of its first entry in the concatenated table, entries, and the device bytes
  * the library keeps for it (table arrays, bucket index, plot, scan work area).  On a replica scan:

@@ -18,7 +18,7 @@ PLOT_CELLS = (SMAX + 1) * (FMAX + 1)
 ABI_SYMBOLS = [
     "hm_last_error", "hm_abi_version", "hm_device_count", "hm_device_info",
     "hm_k_unpack_records", "hm_k_build_bucket_index", "hm_k_pass1_degree", "hm_k_pass2_plot",
-    "hm_k_min_count", "hm_k_find_keys", "hm_pick_bucket_bits", "hm_k_pass2_extract", "hm_scan_extract", "hm_pass2_scratch_bytes",
+    "hm_k_min_count", "hm_k_find_keys", "hm_pick_bucket_bits", "hm_k_pass2_extract", "hm_scan_extract", "hm_scan_extract_path", "hm_pass2_scratch_bytes",
     "hm_k_build_filter", "hm_filter_words", "hm_pick_filter_bits",
     "hm_dev_alloc", "hm_dev_free", "hm_ipc_export", "hm_ipc_open", "hm_ipc_close", "hm_p2p_native_atomics",
     "hm_scan_create", "hm_prewarm", "hm_set_io_threads", "hm_scan_destroy", "hm_scan_examine", "hm_scan_condition", "hm_scan_run", "hm_hetmers_host",
@@ -61,13 +61,22 @@ class SymmShards(C.Structure):
 
 SYMM_ASYMMETRIC, SYMM_OVERFLOW = 1, 2
 PLACE_NOFIT, PLACE_REPLICA, PLACE_SHARDED = 0, 1, 2
-EUNSUPPORTED = -6
+EINVAL, EUNSUPPORTED = -1, -6
 
 
 class PairRec(C.Structure):
     """hm_pair_rec: one line of extract_kmer_pairs' output"""
     _fields_ = [("key_hi", C.c_uint64), ("key_lo", C.c_uint64), ("smudge", C.c_uint32),
                 ("pos", C.c_uint8), ("alt", C.c_uint8), ("pad", C.c_uint16)]
+
+
+class ExtractStats(C.Structure):
+    """hm_extract_stats: route, slices and times of one extraction"""
+    _fields_ = [("path", C.c_int32), ("slices", C.c_int32), ("n_records", C.c_int64),
+                ("ms_kernel", C.c_double), ("ms_copy", C.c_double), ("ms_sort", C.c_double)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
 
 
 class ScanStats(C.Structure):
@@ -142,6 +151,8 @@ def lib():
     L.hm_scan_run_path.argtypes = [vp, i32, vp, C.POINTER(ScanStats)]
     L.hm_scan_is_symmetric.argtypes = [vp]
     L.hm_scan_extract.argtypes = [vp, vp, C.POINTER(C.POINTER(PairRec)), C.POINTER(i64)]
+    L.hm_scan_extract_path.argtypes = [vp, i32, vp, C.POINTER(C.POINTER(PairRec)), C.POINTER(i64),
+                                       C.POINTER(ExtractStats)]
     L.hm_hetmers_host.argtypes = [C.POINTER(HostTable), C.POINTER(i32), i32, vp, C.POINTER(ScanStats)]
     L.hm_scan_download.argtypes = [vp, vp, vp, vp, vp]
     L.hm_scan_create_sharded.argtypes = [C.POINTER(HostTable), C.POINTER(i32), i32, C.POINTER(vp)]

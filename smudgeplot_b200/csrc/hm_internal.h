@@ -33,6 +33,14 @@ typedef struct hm_shard_tabs
 int hm_symm_resolve_sharded(const hm_shard_tabs *tabs, int bits, int idx64, int kmer, void *d_work,
                             const hm_symm_layout *layout, const hm_symm_shards *shards,
                             unsigned long long *d_plot, void *stream);
+/* extract_kmer_pairs from the symmetric scan's candidates, one slice at a time (hm_symm.cu) */
+int64_t hm_symm_extract_slice(const hm_symm_layout *layout);
+int hm_symm_extract(const uint64_t *d_keys, const uint64_t *d_keys_lo, const uint16_t *d_cnt, int64_t n,
+                    const void *d_bucket, const hm_shard_tabs *tabs, int bits, int idx64, int kmer,
+                    void *d_work, const hm_symm_layout *layout, const hm_symm_shards *shards,
+                    const uint16_t *d_pixmap, int64_t c0, int64_t c1, void *stream);
+int hm_symm_extract_fetch(const void *d_work, const hm_symm_layout *layout, hm_pair_rec **buf, int64_t *cap,
+                          int64_t *at, uint64_t *status, void *stream);
 
 #include <cuda_runtime.h>
 /* sharded conditioning (hm_condition.cu) */

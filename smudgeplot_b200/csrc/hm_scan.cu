@@ -65,6 +65,8 @@ struct hm_scan
     int      have_direct;                 /* deg / up / filter allocated and the filter built               */
     int      have_symm;                   /* symmetric-scan work areas allocated, cuts aligned              */
     int      last_path;                   /* HM_PATH_DIRECT / HM_PATH_SYMM of the last run                  */
+    int      symm_ran;                    /* the work areas hold the candidates + Bloom segments of a clean  */
+                                          /*   symmetric scan of the current table (extraction reads them)   */
     int      invalid;                     /* a failed conditioning left the replicas inconsistent            */
     int      sharded;                     /* d[r] holds only entries [d[r].lo, d[r].hi), at local index 0   */
     int      aligned;                     /* sharded: shard r owns the keys in [cut[r], cut[r+1]) (run-aligned) */
@@ -1044,13 +1046,13 @@ extern "C" int hm_scan_condition(hm_scan *s, int ethresh, int do_trim, int do_sy
           HM_CUDA(cudaStreamSynchronize(D->st));
           if (D->symm_work != NULL) { cudaFree(D->symm_work); D->symm_work = NULL; }
         }
-      s->have_symm = 0;
+      s->have_symm = 0; s->symm_ran = 0;
       rc = shard_partition(s,ethresh,do_trim,do_symm);
       if (nels_out) *nels_out = s->n;
       return rc;
     }
   /* everything derived from the old table goes first: work buffers of both paths, the index */
-  s->ran = 0; s->have_direct = 0; s->have_symm = 0;
+  s->ran = 0; s->have_direct = 0; s->have_symm = 0; s->symm_ran = 0;
   for (int g = 0; g < G; g++)
     { DevTable *D = s->d+g;
       HM_CUDA(cudaSetDevice(D->dev));
@@ -1342,6 +1344,7 @@ static int run_symm(hm_scan *s, int64_t *plot, hm_scan_stats *stats, uint64_t *s
   float       ms1 = 0, ms2 = 0, msall = 0;
   if ((rc = ensure_symm(s)) != HM_OK)
     return rc;
+  s->symm_ran = 0;
   hm_shard_tabs tabs;                           /* sharded: pass 2 settles Bloom hits in the owner's arrays */
   memset(&tabs,0,sizeof(tabs));
   for (int g = 0; g < G && s->sharded; g++)
@@ -1434,6 +1437,7 @@ static int run_symm(hm_scan *s, int64_t *plot, hm_scan_stats *stats, uint64_t *s
         cudaEventDestroy(ev[g][k]);
     }
   s->last_path = HM_PATH_SYMM;
+  s->symm_ran  = (*status == 0);
   if (stats != NULL)
     { stats->nels = n; stats->n_gpus = G; stats->bucket_bits = s->bits;
       stats->filter_bits = 0; stats->path = HM_PATH_SYMM;
@@ -1522,9 +1526,11 @@ static int rec_cmp(const void *a, const void *b)
   return ((int) x->alt - (int) y->alt);
 }
 
-/* extract_kmer_pairs' output as a list (PloidyList.c:425-450): needs the incidence array and the
- * recorded partners of a preceding hm_scan_run.  Two launches per GPU: count, then fill.        */
-extern "C" int hm_scan_extract(hm_scan *s, const uint16_t *pixmap, hm_pair_rec **out, int64_t *n_out)
+/* extract_kmer_pairs' output as a list (PloidyList.c:425-450) from the direct passes: needs the
+ * incidence array and the recorded partners (runs the direct passes first if the last run did not).
+ * Two launches per GPU: count, then fill.                                                        */
+static int extract_direct(hm_scan *s, const uint16_t *pixmap, hm_pair_rec **out, int64_t *n_out,
+                          hm_extract_stats *stats)
 { int G = s->ngpu, rc = HM_OK;
   if (s->invalid)
     return hm_set_error(HM_EINVAL,"this scan was left unusable by a failed conditioning");
@@ -1532,6 +1538,7 @@ extern "C" int hm_scan_extract(hm_scan *s, const uint16_t *pixmap, hm_pair_rec *
     return hm_set_error(HM_EUNSUPPORTED,"extract_kmer_pairs needs the direct passes, which a sharded table does not have");
   if ((rc = need_direct_results(s)) != HM_OK)
     return rc;
+  double       t0 = now_ms(), t1, t2;
   int64_t      total = 0, cnts[HM_MAX_GPUS];
   hm_pair_rec *d_out[HM_MAX_GPUS];
   uint16_t    *d_pix[HM_MAX_GPUS];
@@ -1561,6 +1568,7 @@ extern "C" int hm_scan_extract(hm_scan *s, const uint16_t *pixmap, hm_pair_rec *
           if (pass == 0) { cnts[g] = (int64_t) c; total += cnts[g]; }
         }
     }
+  t1 = now_ms();
   hm_pair_rec *host = (hm_pair_rec *) malloc(sizeof(hm_pair_rec)*(size_t) (total > 0 ? total : 1));
   if (host == NULL && rc == HM_OK)
     rc = hm_set_error(HM_ENOMEM,"out of host memory for %lld pair records",(long long) total);
@@ -1578,9 +1586,149 @@ extern "C" int hm_scan_extract(hm_scan *s, const uint16_t *pixmap, hm_pair_rec *
     }
   if (rc != HM_OK)
     { free(host); return rc; }
+  t2 = now_ms();
   qsort(host,(size_t) total,sizeof(hm_pair_rec),rec_cmp);      /* deterministic order */
   *out = host; *n_out = total;
+  if (stats != NULL)
+    { stats->path = HM_PATH_DIRECT; stats->slices = 1; stats->n_records = total;
+      stats->ms_kernel = t1-t0; stats->ms_copy = t2-t1; stats->ms_sort = now_ms()-t2;
+    }
   return HM_OK;
+}
+
+extern "C" int hm_scan_extract(hm_scan *s, const uint16_t *pixmap, hm_pair_rec **out, int64_t *n_out)
+{ return extract_direct(s,pixmap,out,n_out,NULL); }
+
+/* extract_kmer_pairs from the candidates and Bloom segments the symmetric scan left in the work areas
+ * (scanning first if they are not those of a clean scan of the current table).  Every device judges
+ * its own candidates again -- a replica against its replica, a shard with ShardTabs reaching the other
+ * shards -- in slices whose records fit the idle run-head region of its work area; each slice is
+ * copied to the host as it finishes.  The label map goes into the device's plot buffer (the plot of
+ * the last run is on the host already), so nothing is allocated on the device.                      */
+static int extract_symm(hm_scan *s, const uint16_t *pixmap, hm_pair_rec **out, int64_t *n_out,
+                        hm_extract_stats *stats)
+{ int G = s->ngpu, rc = HM_OK;
+  if (!s->sharded && (s->kmer < HM_SYMM_MIN_KMER || !s->symmetric))
+    return hm_set_error(HM_EINVAL,"the table is not strand-symmetric (or k < %d): extraction from the symmetric "
+                                  "scan would not give the reference's pairs",HM_SYMM_MIN_KMER);
+  if (!s->symm_ran)
+    { int64_t *tmp = (int64_t *) malloc(sizeof(int64_t)*HM_PLOT_CELLS);
+      if (tmp == NULL)
+        return hm_set_error(HM_ENOMEM,"out of host memory");
+      rc = hm_scan_run_path(s,HM_PATH_SYMM,tmp,NULL);
+      free(tmp);
+      if (rc != HM_OK)
+        return rc;
+      if (!s->symm_ran)
+        return hm_set_error(HM_EINVAL,"the symmetric scan did not leave its candidates for extraction");
+    }
+  hm_shard_tabs tabs;
+  memset(&tabs,0,sizeof(tabs));
+  for (int g = 0; g < G && s->sharded; g++)
+    { tabs.keys[g] = s->d[g].keys; tabs.keys_lo[g] = s->d[g].keys_lo; tabs.cnt[g] = s->d[g].cnt;
+      tabs.bucket[g] = s->d[g].bucket; tabs.n[g] = s->d[g].hi-s->d[g].lo;
+    }
+  int64_t  nc[HM_MAX_GPUS], cur[HM_MAX_GPUS], slice[HM_MAX_GPUS];
+  float    ms_k[HM_MAX_GPUS];
+  cudaEvent_t ev[HM_MAX_GPUS][2];
+  uint16_t *d_pix[HM_MAX_GPUS];
+  for (int g = 0; g < G; g++)
+    { DevTable *D = s->d+g;
+      uint64_t  n_cand = 0, st = 0;
+      HM_CUDA(cudaSetDevice(D->dev));
+      HM_CUDA(cudaEventCreate(&ev[g][0]));
+      HM_CUDA(cudaEventCreate(&ev[g][1]));
+      d_pix[g] = (uint16_t *) D->plot;
+      HM_CUDA(cudaMemcpyAsync(d_pix[g],pixmap,sizeof(uint16_t)*HM_PLOT_CELLS,cudaMemcpyHostToDevice,D->st));
+      if ((rc = hm_symm_status(D->symm_work,&D->symm_layout,&n_cand,&st,D->st)) != HM_OK)
+        return rc;
+      nc[g] = (int64_t) n_cand < D->symm_layout.cand_cap ? (int64_t) n_cand : D->symm_layout.cand_cap;
+      cur[g] = 0; ms_k[g] = 0;
+      slice[g] = hm_symm_extract_slice(&D->symm_layout);
+    }
+  double       t_copy = 0;
+  int64_t      at = 0, cap = 0;
+  int          slices = 0;
+  uint64_t     status = 0;
+  hm_pair_rec *host = NULL;
+  for (int more = 1; more && rc == HM_OK; )
+    { more = 0;
+      for (int g = 0; g < G && rc == HM_OK; g++)           /* one slice on every device that has candidates left */
+        { DevTable *D = s->d+g;
+          if (cur[g] >= nc[g]) continue;
+          int64_t c1 = cur[g]+slice[g] < nc[g] ? cur[g]+slice[g] : nc[g];
+          cudaSetDevice(D->dev);
+          cudaEventRecord(ev[g][0],D->st);
+          rc = hm_symm_extract(D->keys,D->keys_lo,D->cnt,s->sharded ? D->hi-D->lo : s->n,D->bucket,
+                               s->sharded ? &tabs : NULL,s->bits,s->idx64,s->kmer,D->symm_work,&D->symm_layout,
+                               G > 1 ? &s->ssh[g] : NULL,d_pix[g],cur[g],c1,D->st);
+          cudaEventRecord(ev[g][1],D->st);
+          s->launches += 1;
+          slices += 1;
+        }
+      for (int g = 0; g < G && rc == HM_OK; g++)           /* ... and its records to the host */
+        { DevTable *D = s->d+g;
+          if (cur[g] >= nc[g]) continue;
+          float    ms = 0;
+          uint64_t st = 0;
+          cudaSetDevice(D->dev);
+          cudaError_t e = cudaEventSynchronize(ev[g][1]);
+          if (e != cudaSuccess) { rc = hm_cuda_fail(e,"extract_kernel"); break; }
+          cudaEventElapsedTime(&ms,ev[g][0],ev[g][1]);
+          ms_k[g] += ms;
+          double t = now_ms();
+          rc = hm_symm_extract_fetch(D->symm_work,&D->symm_layout,&host,&cap,&at,&st,D->st);
+          t_copy += now_ms()-t;
+          status |= st;
+          cur[g] += slice[g];
+          if (cur[g] < nc[g]) more = 1;
+        }
+    }
+  for (int g = 0; g < G; g++)
+    { cudaSetDevice(s->d[g].dev);
+      cudaEventDestroy(ev[g][0]); cudaEventDestroy(ev[g][1]);
+    }
+  if (rc == HM_OK && status != 0)
+    { s->symm_ran = 0;                    /* judged again, a candidate came out differently: nothing is trusted */
+      rc = hm_set_error(HM_EINVAL,"extraction from the symmetric scan failed its own checks (status %llu)",
+                        (unsigned long long) status);
+    }
+  if (rc != HM_OK)
+    { free(host); return rc; }
+  if (host == NULL && (host = (hm_pair_rec *) malloc(sizeof(hm_pair_rec))) == NULL)
+    return hm_set_error(HM_ENOMEM,"out of host memory");
+  double t = now_ms();
+  qsort(host,(size_t) at,sizeof(hm_pair_rec),rec_cmp);         /* the order of hm_scan_extract */
+  *out = host; *n_out = at;
+  if (stats != NULL)
+    { float mk = 0;
+      for (int g = 0; g < G; g++) if (ms_k[g] > mk) mk = ms_k[g];
+      stats->path = HM_PATH_SYMM; stats->slices = slices; stats->n_records = at;
+      stats->ms_kernel = mk; stats->ms_copy = t_copy; stats->ms_sort = now_ms()-t;
+    }
+  return HM_OK;
+}
+
+extern "C" int hm_scan_extract_path(hm_scan *s, int path, const uint16_t *pixmap, hm_pair_rec **out,
+                                    int64_t *n_out, hm_extract_stats *stats)
+{ if (s == NULL || pixmap == NULL || out == NULL || n_out == NULL)
+    return hm_set_error(HM_EINVAL,"hm_scan_extract_path: bad arguments");
+  if (s->invalid)
+    return hm_set_error(HM_EINVAL,"this scan was left unusable by a failed conditioning");
+  if (path != HM_PATH_AUTO && path != HM_PATH_DIRECT && path != HM_PATH_SYMM)
+    return hm_set_error(HM_EINVAL,"hm_scan_extract_path: unknown path %d",path);
+  if (stats != NULL)
+    memset(stats,0,sizeof(*stats));
+  if (path == HM_PATH_AUTO)                       /* the path hm_scan_run takes */
+    { const char *e = getenv("HETMERS_PATH");
+      if (s->sharded)                             path = HM_PATH_SYMM;
+      else if (e != NULL && strcmp(e,"direct") == 0) path = HM_PATH_DIRECT;
+      else if (e != NULL && strcmp(e,"symm") == 0)   path = HM_PATH_SYMM;
+      else path = (s->symmetric && s->kmer >= HM_SYMM_MIN_KMER) ? HM_PATH_SYMM : HM_PATH_DIRECT;
+    }
+  if (path == HM_PATH_DIRECT)
+    return extract_direct(s,pixmap,out,n_out,stats);
+  return extract_symm(s,pixmap,out,n_out,stats);
 }
 
 extern "C" int hm_hetmers_host(const hm_host_table *t, const int *dev, int n_gpus,

@@ -1250,29 +1250,119 @@ __device__ __forceinline__ void count_pair(uint32_t *tile, unsigned long long *_
     atomicAdd(plot + s*HM_PLOT_W + m, (unsigned long long) wgt);
 }
 
-/* Candidates whose Bloom look-up misses (~95 %) are counted at once.  The others need the exact
+/* What pass 2 does with a candidate judged to be an isolated pair (take() is called by the lanes that
+ * hold one):
+ *   PlotSink    counts it into the plot (resolve_kernel, resolve_sharded_kernel)
+ *   RecordSink  writes extract_kmer_pairs' records of it (extract_kernel, extract_sharded_kernel)
+ * first() / last() pick the candidates [first, min(count, last)) the kernel judges.                   */
+struct PlotSink
+  { unsigned long long *plot;
+    int kmer;
+    __device__ __forceinline__ int64_t first() const { return 0; }
+    __device__ __forceinline__ int64_t last(int64_t nc) const { return nc; }
+    __device__ __forceinline__ void begin() const
+    { extern __shared__ uint32_t tile[];
+      for (int t = threadIdx.x; t < RV_TS*RV_TM; t += blockDim.x)
+        tile[t] = 0;
+      __syncthreads();
+    }
+    __device__ __forceinline__ void take(uint64_t, uint64_t, uint64_t meta) const
+    { extern __shared__ uint32_t tile[];
+      count_pair(tile,plot,meta,kmer);
+    }
+    __device__ __forceinline__ void end() const
+    { extern __shared__ uint32_t tile[];
+      __syncthreads();
+      for (int t = threadIdx.x; t < RV_TS*RV_TM; t += blockDim.x)
+        { uint32_t v = tile[t];
+          if (v != 0)
+            atomicAdd(plot + (t/RV_TM)*HM_PLOT_W + (t%RV_TM), (unsigned long long) v);
+        }
+    }
+  };
+
+/* extract_kmer_pairs' records of one isolated candidate x < y (differing at p >= k/2, x's base bx <
+ * y's base by), when its pixel carries a label -- what the reference prints for the pair and for its
+ * mirror image (PloidyList.c:432-447), which the direct passes find as a pair of its own:
+ *   the pair         cx < cy: y with alt bx, else (a tie too) x with alt by;             pos p
+ *   the mirror       (rc y, rc x): rc y is the lower member (3-by < 3-bx at k-1-p) and has count cy,
+ *                    so cy < cx: rc x with alt 3-by, else (a tie too) rc y with alt 3-bx; pos k-1-p
+ * The mirror is left out at the middle base of an odd k (2p == k-1), where it is found as a candidate
+ * itself -- count_pair's weight of 1 -- so n records == plot[pixmap > 0].sum().  Records are appended
+ * with one global atomic per warp and call (ballot + prefix over the lanes that hold an isolated pair:
+ * the active mask).  A slice of the candidates yields at most 2 records each, so `cap` is never reached.          */
+template <int KW>
+struct RecordSink
+  { const uint16_t *pixmap;
+    hm_pair_rec *out;
+    unsigned long long *out_n, *status, cap;
+    int64_t c0, c1;
+    int kmer;
+    __device__ __forceinline__ int64_t first() const { return c0; }
+    __device__ __forceinline__ int64_t last(int64_t nc) const { return nc < c1 ? nc : c1; }
+    __device__ __forceinline__ void begin() const {}
+    __device__ __forceinline__ void end() const {}
+    __device__ __forceinline__ void put(unsigned long long at, uint64_t h, uint64_t l, uint32_t lab, int pos, int alt) const
+    { if (at >= cap)
+        { atomicOr(status,SY_STATUS_OVERFLOW); return; }
+      hm_pair_rec r;
+      r.key_hi = h; r.key_lo = l; r.smudge = lab; r.pos = (uint8_t) pos; r.alt = (uint8_t) alt; r.pad = 0;
+      out[at] = r;
+    }
+    __device__ __forceinline__ void take(uint64_t x, uint64_t xl, uint64_t meta) const
+    { const int cx = (int) (meta & 0xffff), cy = (int) ((meta >> 16) & 0xffff);
+      const int p  = (int) ((meta >> 32) & 0xff), by = (int) ((meta >> 40) & 3);
+      const uint32_t lab = __ldg(pixmap + (cx+cy)*HM_PLOT_W + (cx < cy ? cx : cy));
+      const bool     one = (lab != 0), two = one && (2*p != kmer-1);
+      const unsigned m  = __activemask();
+      const unsigned b1 = __ballot_sync(m,one), b2 = __ballot_sync(m,two);
+      if (b1 == 0)
+        return;
+      const int      lane = threadIdx.x & 31, lead = __ffs((int) m)-1;
+      const unsigned lt   = (1u << lane) - 1;
+      unsigned long long at = 0;
+      if (lane == lead)
+        at = atomicAdd(out_n,(unsigned long long) (__popc(b1)+__popc(b2)));
+      at = __shfl_sync(m,at,lead) + (unsigned long long) (__popc(b1 & lt) + __popc(b2 & lt));
+      if (!one)
+        return;
+      const int bx = base_at<KW>(x,xl,p);
+      uint64_t  y = x, yl = xl;
+      set_base<KW>(y,yl,p,by);
+      if (cx < cy) put(at,y,yl,lab,p,bx);
+      else         put(at,x,xl,lab,p,by);
+      if (!two)
+        return;
+      uint64_t rx, rxl, ry, ryl;
+      revcomp_kmer<KW>(x,xl,kmer,rx,rxl);
+      ry = rx; ryl = rxl;
+      set_base<KW>(ry,ryl,kmer-1-p,3-by);
+      if (cy < cx) put(at+1,rx,rxl,lab,kmer-1-p,3-by);
+      else         put(at+1,ry,ryl,lab,kmer-1-p,3-bx);
+    }
+  };
+
+/* Candidates whose Bloom look-up misses (~95 %) are settled at once.  The others need the exact
  * answer -- bucket offsets, keys, counts: three dependent random accesses -- and a warp in which one
  * lane does that stalls all 32: they are parked in a per-warp queue and settled 32 at a time, every
  * lane busy.  RV_ILP candidates per thread and trip keep that many record / Bloom loads in flight
  * (the kernel is bound by the latency of record -> Bloom word, not by bytes or instructions).         */
-template <typename IdxT, int KW, typename Tabs>
+template <typename IdxT, int KW, typename Tabs, typename Sink>
 __device__ __forceinline__ void resolve_body(const uint64_t *__restrict__ keys, const uint64_t *__restrict__ keys_lo,
                                              const uint16_t *__restrict__ cnt, int64_t n, const IdxT *__restrict__ bucket,
-                                             int bshift, int kmer, const SymmView &W, const Tabs &T,
-                                             unsigned long long *__restrict__ plot)
-{ extern __shared__ uint32_t tile[];
-  __shared__ uint32_t s_q[RV_THREADS/32][32*(RV_ILP+1)];
+                                             int bshift, int kmer, const SymmView &W, const Tabs &T, const Sink &sink)
+{ __shared__ uint32_t s_q[RV_THREADS/32][32*(RV_ILP+1)];
   const unsigned FULL = 0xffffffffu;
   const int      lane = threadIdx.x & 31;
   const unsigned lt   = (1u << lane) - 1;
   uint32_t *q  = s_q[threadIdx.x >> 5];
   int       qn = 0;
-  for (int t = threadIdx.x; t < RV_TS*RV_TM; t += blockDim.x)
-    tile[t] = 0;
-  __syncthreads();
+  sink.begin();
   unsigned long long ncl = *W.cand_n;
   if (ncl > W.cand_cap) ncl = W.cand_cap;
-  const int64_t nc     = (int64_t) ncl;
+  const int64_t c0     = sink.first();
+  const int64_t nc     = sink.last((int64_t) ncl) - c0;
+  const uint64_t *ckey = W.cand_key + c0, *clo = W.cand_lo + c0, *cmeta = W.cand_meta + c0;
   const int64_t stride = (int64_t) gridDim.x * blockDim.x;
   const int64_t first  = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
   for (uint32_t it = 0; first-lane + (int64_t) it*RV_ILP*stride < nc; it++)
@@ -1285,9 +1375,9 @@ __device__ __forceinline__ void resolve_body(const uint64_t *__restrict__ keys, 
           ok[u] = (i < nc);
           x[u] = 0; xl[u] = 0; meta[u] = 0;
           if (ok[u])
-            { x[u] = ld_stream(W.cand_key+i);
-              if (KW == 2) xl[u] = ld_stream(W.cand_lo+i);
-              meta[u] = ld_stream(W.cand_meta+i);
+            { x[u] = ld_stream(ckey+i);
+              if (KW == 2) xl[u] = ld_stream(clo+i);
+              meta[u] = ld_stream(cmeta+i);
             }
         }
 #pragma unroll
@@ -1312,7 +1402,7 @@ __device__ __forceinline__ void resolve_body(const uint64_t *__restrict__ keys, 
       for (int u = 0; u < RV_ILP; u++)
         { const bool hit = ok[u] && ((va[u] & ba[u]) == ba[u] || (vb[u] & bb[u]) == bb[u]);
           if (ok[u] && !hit)
-            count_pair(tile,plot,meta[u],kmer);
+            sink.take(x[u],xl[u],meta[u]);
           const unsigned bal = __ballot_sync(FULL,hit);
           if (hit)
             q[qn + __popc(bal & lt)] = ((it*RV_ILP+u) << 5) | (uint32_t) lane;
@@ -1324,24 +1414,19 @@ __device__ __forceinline__ void resolve_body(const uint64_t *__restrict__ keys, 
           const uint32_t e = q[qn+lane];
           __syncwarp();
           const int64_t j = first-lane + (int64_t) (e & 31) + (int64_t) (e >> 5)*stride;
-          const uint64_t xx = W.cand_key[j], xxl = KW == 2 ? W.cand_lo[j] : 0, mm = W.cand_meta[j];
+          const uint64_t xx = ckey[j], xxl = KW == 2 ? clo[j] : 0, mm = cmeta[j];
           if (judge_candidate<IdxT,KW,true>(keys,keys_lo,cnt,n,bucket,bshift,kmer,W,T,xx,xxl,mm) == 0)
-            count_pair(tile,plot,mm,kmer);
+            sink.take(xx,xxl,mm);
         }
     }
   if (lane < qn)
     { const uint32_t e = q[lane];
       const int64_t j = first-lane + (int64_t) (e & 31) + (int64_t) (e >> 5)*stride;
-      const uint64_t xx = W.cand_key[j], xxl = KW == 2 ? W.cand_lo[j] : 0, mm = W.cand_meta[j];
+      const uint64_t xx = ckey[j], xxl = KW == 2 ? clo[j] : 0, mm = cmeta[j];
       if (judge_candidate<IdxT,KW,true>(keys,keys_lo,cnt,n,bucket,bshift,kmer,W,T,xx,xxl,mm) == 0)
-        count_pair(tile,plot,mm,kmer);
+        sink.take(xx,xxl,mm);
     }
-  __syncthreads();
-  for (int t = threadIdx.x; t < RV_TS*RV_TM; t += blockDim.x)
-    { uint32_t v = tile[t];
-      if (v != 0)
-        atomicAdd(plot + (t/RV_TM)*HM_PLOT_W + (t%RV_TM), (unsigned long long) v);
-    }
+  sink.end();
 }
 
 template <typename IdxT, int KW>
@@ -1349,14 +1434,32 @@ __global__ void __launch_bounds__(RV_THREADS,RV_CTAS_PER_SM)
 resolve_kernel(const uint64_t *__restrict__ keys, const uint64_t *__restrict__ keys_lo,
                const uint16_t *__restrict__ cnt, int64_t n, const IdxT *__restrict__ bucket, int bshift,
                int kmer, const SymmView W, unsigned long long *__restrict__ plot)
-{ resolve_body<IdxT,KW>(keys,keys_lo,cnt,n,bucket,bshift,kmer,W,NoTabs(),plot); }
+{ resolve_body<IdxT,KW>(keys,keys_lo,cnt,n,bucket,bshift,kmer,W,NoTabs(),PlotSink{plot,kmer}); }
 
 /* pass 2 of a sharded scan: the same, with every Bloom hit settled in the owner's arrays */
 template <typename IdxT, int KW>
 __global__ void __launch_bounds__(RV_THREADS,RV_CTAS_PER_SM)
 resolve_sharded_kernel(int bshift, int kmer, const SymmView W, const ShardTabs T, unsigned long long *__restrict__ plot)
 { resolve_body<IdxT,KW>((const uint64_t *) NULL,(const uint64_t *) NULL,(const uint16_t *) NULL,(int64_t) 0,
-                        (const IdxT *) NULL,bshift,kmer,W,T,plot);
+                        (const IdxT *) NULL,bshift,kmer,W,T,PlotSink{plot,kmer});
+}
+
+/* extract_kmer_pairs from the symmetric scan: pass 2 over the candidates [c0, c1) of the last run
+ * scan, isolated pairs written as records (RecordSink) instead of counted.  The record sink keeps the
+ * candidates' keys live across the loop, which does not fit the 64 registers of two CTAs per SM
+ * without spilling: one CTA per SM (the kernel runs once per extraction, not once per scan).       */
+template <typename IdxT, int KW>
+__global__ void __launch_bounds__(RV_THREADS,1)
+extract_kernel(const uint64_t *__restrict__ keys, const uint64_t *__restrict__ keys_lo,
+               const uint16_t *__restrict__ cnt, int64_t n, const IdxT *__restrict__ bucket, int bshift,
+               int kmer, const SymmView W, const RecordSink<KW> R)
+{ resolve_body<IdxT,KW>(keys,keys_lo,cnt,n,bucket,bshift,kmer,W,NoTabs(),R); }
+
+template <typename IdxT, int KW>
+__global__ void __launch_bounds__(RV_THREADS,1)
+extract_sharded_kernel(int bshift, int kmer, const SymmView W, const ShardTabs T, const RecordSink<KW> R)
+{ resolve_body<IdxT,KW>((const uint64_t *) NULL,(const uint64_t *) NULL,(const uint16_t *) NULL,(int64_t) 0,
+                        (const IdxT *) NULL,bshift,kmer,W,T,R);
 }
 
 template <typename IdxT, int KW>
@@ -1443,6 +1546,99 @@ int hm_symm_resolve_sharded(const hm_shard_tabs *tabs, int bits, int idx64, int 
     bloom_window(st,NULL,0,0);
   if (e != cudaSuccess)
     return hm_cuda_fail(e,"resolve_sharded_kernel");
+  return HM_OK;
+}
+
+/* ----------------------------------------------------------- pass 2, extract variant -- */
+
+/* The records of an extraction are staged in the run-head region of the work area (idle once pass 1 is
+ * done; the next run scan starts it afresh) and counted in header word 3: 8*runs_cap bytes hold cap =
+ * 8*runs_cap/24 records, enough for the records of cap/2 candidates -- one slice.                    */
+#define SY_HDR_RECORDS 3
+
+int64_t hm_symm_extract_slice(const hm_symm_layout *layout)
+{ return (8*layout->runs_cap / (int64_t) sizeof(hm_pair_rec)) / 2; }
+
+template <typename IdxT, int KW>
+static cudaError_t launch_extract(const uint64_t *keys, const uint64_t *keys_lo, const uint16_t *cnt, int64_t n,
+                                  const void *bucket, const hm_shard_tabs *tabs, int bits, int kmer,
+                                  const SymmView &W, const RecordSink<KW> &R, cudaStream_t st)
+{ int dev = 0, sms = 148;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&sms,cudaDevAttrMultiProcessorCount,dev);
+  int64_t want = (R.c1-R.c0+RV_THREADS-1)/RV_THREADS;
+  int     grid = (int) (want < sms ? (want > 0 ? want : 1) : sms);
+  if (tabs != NULL)
+    extract_sharded_kernel<IdxT,KW><<<grid,RV_THREADS,0,st>>>(64-bits,kmer,W,*tabs,R);
+  else
+    extract_kernel<IdxT,KW><<<grid,RV_THREADS,0,st>>>(keys,keys_lo,cnt,n,(const IdxT *) bucket,64-bits,kmer,W,R);
+  return cudaGetLastError();
+}
+
+/* extract_kmer_pairs' records of the candidates [c0, c1) (c1-c0 <= hm_symm_extract_slice) of the last
+ * symmetric scan on this work area, labelled by d_pixmap (uint16[HM_PLOT_CELLS] on the device): into the
+ * run-head region, count in header word 3 (both read back with hm_symm_extract_fetch).  tabs != NULL: a
+ * sharded table (keys .. bucket unused), Bloom hits are settled in the owning shard's arrays.          */
+int hm_symm_extract(const uint64_t *d_keys, const uint64_t *d_keys_lo, const uint16_t *d_cnt, int64_t n,
+                    const void *d_bucket, const hm_shard_tabs *tabs, int bits, int idx64, int kmer,
+                    void *d_work, const hm_symm_layout *layout, const hm_symm_shards *shards,
+                    const uint16_t *d_pixmap, int64_t c0, int64_t c1, void *stream)
+{ if (kmer < HM_SYMM_MIN_KMER || kmer > HM_MAX_KMER || d_work == NULL || layout == NULL || d_pixmap == NULL ||
+      c0 < 0 || c1 < c0 || c1-c0 > hm_symm_extract_slice(layout))
+    return hm_set_error(HM_EINVAL,"symm_extract: bad arguments");
+  if (tabs == NULL && (kmer > 32) != (d_keys_lo != NULL))
+    return hm_set_error(HM_EINVAL,"symm_extract: second key word array %s for k=%d",d_keys_lo ? "given" : "missing",kmer);
+  cudaStream_t st = (cudaStream_t) stream;
+  SymmView W = make_view(d_work,layout,shards);
+  uint8_t *b = (uint8_t *) d_work;
+  unsigned long long *recs_n = W.cand_n + SY_HDR_RECORDS;
+  HM_CUDA(cudaMemsetAsync(recs_n,0,sizeof(unsigned long long),st));
+  if (l2_persist())
+    bloom_window(st,W.bloom,sizeof(uint32_t)*(size_t) W.seg_words*(size_t) W.n_seg,1);
+  cudaError_t e;
+  if (kmer <= 32)
+    { RecordSink<1> R = { d_pixmap,(hm_pair_rec *) (b + layout->off_runs),recs_n,W.status,
+                          (unsigned long long) (2*hm_symm_extract_slice(layout)),c0,c1,kmer };
+      e = idx64 ? launch_extract<uint64_t,1>(d_keys,NULL,d_cnt,n,d_bucket,tabs,bits,kmer,W,R,st)
+                : launch_extract<uint32_t,1>(d_keys,NULL,d_cnt,n,d_bucket,tabs,bits,kmer,W,R,st);
+    }
+  else
+    { RecordSink<2> R = { d_pixmap,(hm_pair_rec *) (b + layout->off_runs),recs_n,W.status,
+                          (unsigned long long) (2*hm_symm_extract_slice(layout)),c0,c1,kmer };
+      e = idx64 ? launch_extract<uint64_t,2>(d_keys,d_keys_lo,d_cnt,n,d_bucket,tabs,bits,kmer,W,R,st)
+                : launch_extract<uint32_t,2>(d_keys,d_keys_lo,d_cnt,n,d_bucket,tabs,bits,kmer,W,R,st);
+    }
+  if (l2_persist())
+    bloom_window(st,NULL,0,0);
+  if (e != cudaSuccess)
+    return hm_cuda_fail(e,tabs != NULL ? "extract_sharded_kernel" : "extract_kernel");
+  return HM_OK;
+}
+
+/* after hm_symm_extract on `stream`: appends its records to the host array *buf (malloc'ed; *cap
+ * records, *at in use; grown as needed) and ORs the work area's status word into *status (synchronises) */
+int hm_symm_extract_fetch(const void *d_work, const hm_symm_layout *layout, hm_pair_rec **buf, int64_t *cap,
+                          int64_t *at, uint64_t *status, void *stream)
+{ uint64_t h[4] = {0,0,0,0};
+  cudaStream_t st = (cudaStream_t) stream;
+  HM_CUDA(cudaMemcpyAsync(h,(const uint8_t *) d_work + layout->off_header,sizeof(h),cudaMemcpyDeviceToHost,st));
+  HM_CUDA(cudaStreamSynchronize(st));
+  const int64_t room = 2*hm_symm_extract_slice(layout);
+  const int64_t m    = (int64_t) h[SY_HDR_RECORDS] < room ? (int64_t) h[SY_HDR_RECORDS] : room;
+  *status |= h[1];
+  if (m <= 0)
+    return HM_OK;
+  if (*at + m > *cap)
+    { int64_t nc = *cap*2 > *at+m ? *cap*2 : *at+m;
+      hm_pair_rec *nb = (hm_pair_rec *) realloc(*buf,sizeof(hm_pair_rec)*(size_t) nc);
+      if (nb == NULL)
+        return hm_set_error(HM_ENOMEM,"out of host memory for %lld pair records",(long long) nc);
+      *buf = nb; *cap = nc;
+    }
+  HM_CUDA(cudaMemcpyAsync(*buf + *at,(const uint8_t *) d_work + layout->off_runs,sizeof(hm_pair_rec)*(size_t) m,
+                          cudaMemcpyDeviceToHost,st));
+  HM_CUDA(cudaStreamSynchronize(st));
+  *at += m;
   return HM_OK;
 }
 

@@ -156,14 +156,23 @@ class Scan:
         _lib.check(self._L.hm_scan_run_path(self._h, self.PATHS[path], plot.ctypes.data, C.byref(st)))
         return plot.reshape(_lib.SMAX + 1, _lib.PLOT_W), st.as_dict()
 
-    def extract(self, pixmap: np.ndarray):
-        """pair list of extract_kmer_pairs (after run()): pixmap uint16[1001,501], label 0 = none;
-        -> structured array (key_hi, key_lo, smudge, pos, alt) sorted by (smudge, k-mer)"""
+    def extract(self, pixmap: np.ndarray, path: str | None = None, stats: bool = False):
+        """pair list of extract_kmer_pairs: pixmap uint16[1001,501], label 0 = none; -> structured array
+        (key_hi, key_lo, smudge, pos, alt) sorted by (smudge, k-mer).  path=None: hm_scan_extract (the
+        direct passes, run first if the last run was not theirs); "auto" / "direct" / "symm":
+        hm_scan_extract_path ("symm" re-judges the symmetric scan's candidates and works on sharded
+        tables; "auto" takes the route run() takes).  stats=True: -> (records, stats dict)"""
         pm = np.ascontiguousarray(pixmap, dtype=np.uint16).reshape(-1)
         assert pm.size == _lib.PLOT_CELLS
         out = C.POINTER(_lib.PairRec)()
         n = C.c_int64()
-        _lib.check(self._L.hm_scan_extract(self._h, pm.ctypes.data, C.byref(out), C.byref(n)))
+        st = _lib.ExtractStats()
+        if path is None:
+            _lib.check(self._L.hm_scan_extract(self._h, pm.ctypes.data, C.byref(out), C.byref(n)))
+            st.path, st.slices, st.n_records = 1, 1, n.value
+        else:
+            _lib.check(self._L.hm_scan_extract_path(self._h, self.PATHS[path], pm.ctypes.data, C.byref(out),
+                                                    C.byref(n), C.byref(st)))
         dt = np.dtype([("key_hi", "<u8"), ("key_lo", "<u8"), ("smudge", "<u4"), ("pos", "u1"), ("alt", "u1"),
                        ("pad", "<u2")])
         arr = np.empty(n.value, dtype=dt)
@@ -172,7 +181,7 @@ class Scan:
         libc = C.CDLL(None)
         libc.free.argtypes = [C.c_void_p]
         libc.free(out)
-        return arr
+        return (arr, st.as_dict()) if stats else arr
 
     def download(self, deg: bool = True):
         """-> (keys, cnt, deg) of the device table; a sharded table gives the concatenation of its shards

@@ -522,11 +522,16 @@ int main(int argc, char *argv[])
     die_hm();
   t_scan = wall_ms();
 #ifdef EXTRACT_PAIRS
-  hm_pair_rec *REC = NULL;
-  int64_t      NREC = 0;
-  int          KMER = hm_table_view(T)->kmer;
-  if (hm_scan_extract(S,PIXMAP,&REC,&NREC) != HM_OK)
+  //  The isolated pairs of the labelled pixels, by the route the scan took: from the symmetric scan's
+  //  candidates (any placement, sharded included) or from the direct passes
+  hm_pair_rec     *REC = NULL;
+  int64_t          NREC = 0;
+  int              KMER = hm_table_view(T)->kmer;
+  hm_extract_stats XST;
+  double           t_extract = wall_ms();
+  if (hm_scan_extract_path(S,HM_PATH_AUTO,PIXMAP,&REC,&NREC,&XST) != HM_OK)
     die_hm();
+  t_extract = wall_ms()-t_extract;
 #endif
   //  (the device-resident table is not torn down: the process is about to end, and destroying the CUDA
   //   context by hand costs ~0.1 s of wall clock for nothing)
@@ -540,6 +545,13 @@ int main(int argc, char *argv[])
         }
       fprintf(stderr,"], ");
     }
+#ifdef EXTRACT_PAIRS
+  if (getenv("HETMERS_STATS") != NULL)
+    fprintf(stderr,"\"extract\": {\"path\": \"%s\", \"pairs\": %lld, \"slices\": %d, \"ms_kernel\": %.3f, "
+                   "\"ms_copy\": %.3f, \"ms_sort\": %.3f, \"wall_ms\": %.1f}, ",
+            XST.path == HM_PATH_SYMM ? "symmetric" : "direct",(long long) XST.n_records,XST.slices,
+            XST.ms_kernel,XST.ms_copy,XST.ms_sort,t_extract);
+#endif
   if (getenv("HETMERS_STATS") != NULL)
     fprintf(stderr,"\"nels\": %lld, \"n_gpus\": %d, \"path\": \"%s\", \"bucket_bits\": %d, \"ms_load\": %.3f, "
                    "\"ms_pass1\": %.3f, \"ms_pass2\": %.3f, \"ms_scan\": %.3f, \"kernel_launches\": %lld, "
